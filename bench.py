@@ -283,6 +283,8 @@ def run_b200(args):
         dist.all_reduce(t, op=dist.ReduceOp.MAX)
     ms = float(t.item())
     value = world * chains * args.steps / (ms * 1e-3)
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, eng)
 
     # ---- end to end through the public API with host buffers -----------------
     pinned_events = torch.empty(len(events) * 48, dtype=torch.uint8, pin_memory=True)
@@ -588,16 +590,17 @@ def cpp_tree_leg(chains, events_n):
     TTree::Fill per chain -- and StepMany() without one."""
     import re
     import subprocess
+    import tempfile
     libdir = os.path.join(ROOT, "root-simple-mcmc_b200", "smcmc_b200")
-    exe = os.path.join(ROOT, "tests", "cpp", "_build", "simple_mcmc")
     src = os.path.join(ROOT, "tests", "cpp", "simple_mcmc.cc")
     try:
-        os.makedirs(os.path.dirname(exe), exist_ok=True)
-        if not os.path.exists(exe) or os.path.getmtime(exe) < os.path.getmtime(src):
+        # compiled outside the source tree, which may be read-only
+        with tempfile.TemporaryDirectory(prefix="smcmc_bench_") as tmp:
+            exe = os.path.join(tmp, "simple_mcmc")
             subprocess.run(["g++", "-std=c++17", "-O2", "-I", os.path.join(ROOT, "include"), "-o", exe, src,
                             "-L", libdir, "-lsmcmc_b200", "-Wl,-rpath," + libdir], check=True)
-        r = subprocess.run([exe, "tree", str(chains), "10", str(max(1, events_n // 30))], capture_output=True, text=True,
-                           check=True, timeout=600)
+            r = subprocess.run([exe, "tree", str(chains), "10", str(max(1, events_n // 30))], capture_output=True,
+                               text=True, check=True, timeout=600)
         m = re.search(r"events (\d+) ms_per_step_plain (\S+) ms_per_step_tree (\S+) full_save_ms (\S+) entries (\d+)", r.stdout)
         plain, tree = float(m.group(2)), float(m.group(3))
         return {"value": chains / (tree * 1e-3), "unit": "steps/s", "ms_per_step_with_tree": tree,
@@ -607,6 +610,28 @@ def cpp_tree_leg(chains, events_n):
                         "include/smcmc_tree.h; ROOT is not installed): one TTree::Fill per chain and step on the host"}
     except Exception as exc:                          # reported, never fatal for the headline line
         return {"unavailable": "%s: %s" % (type(exc).__name__, exc)}
+
+
+DUMP_MAX_CHAINS = 262144          # x (2 x 9 + 3) float64 per chain = 44 MB
+
+
+def dump_outputs(out_dir, eng):
+    """What the last timed step left for a caller of the step path, one .npy per array: every
+    chain's accepted point and likelihood, the point it proposed and its likelihood, and its
+    proposal step size (4096 chains: 0.7 MB in float64).  Above DUMP_MAX_CHAINS chains a fixed
+    seeded sample of them is written, with their indices in chain_index.npy.  At a fixed
+    --steps and --warmup the inputs and the number of steps taken (max(--warmup, 3) + --steps)
+    are the same on every run, so two builds can be compared array by array."""
+    os.makedirs(out_dir, exist_ok=True)
+    eng.sync()
+    keep = slice(None)
+    if eng.chains > DUMP_MAX_CHAINS:
+        keep = np.sort(np.random.default_rng(0).choice(eng.chains, DUMP_MAX_CHAINS, replace=False))
+        np.save(os.path.join(out_dir, "chain_index.npy"), keep.astype(np.float64))
+    for name, field in (("accepted_points", "accepted"), ("accepted_llh", "accepted_llh"),
+                        ("proposed_points", "proposed"), ("proposed_llh", "proposed_llh"),
+                        ("sigma", "sigma")):
+        np.save(os.path.join(out_dir, name + ".npy"), eng.get(field)[keep].astype(np.float64))
 
 
 _RESULT_OUT = None
@@ -639,7 +664,15 @@ def main():
     ap.add_argument("--c4-chains", type=int, default=16384, help="--config c4: chains per GPU")
     ap.add_argument("--config", default="c2", choices=["c1", "c2", "c3", "c4"],
                     help="which BASELINE.json config to measure (default c2, the headline one)")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write the chains' state after the last step as DIR/<name>.npy "
+                         "(default config, rank 0's chains); fixed by --steps and --warmup, where any --warmup "
+                         "below 3 runs 3 warm-up steps")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and (args.config != "c2" or args.impl != "b200"):
+        ap.error("--dump-outputs is implemented for the default config of the b200 arm")
     # stdout carries exactly ONE line, the JSON result: anything else that writes to file
     # descriptor 1 (NCCL prints its version banner there when the first communicator is
     # made, child processes inherit it) is sent to stderr; emit() writes to the saved descriptor

@@ -123,8 +123,6 @@ def load(which):
         lib.ref_dummy_matrices.argtypes = [vp, vp]
         lib.ref_ex2_generate.restype = ctypes.c_long
         lib.ref_ex2_generate.argtypes = [ctypes.c_ulong, ci, ci, cd, vp, ctypes.c_long, vp]
-        lib.ref_shim_linalg.restype = ci
-        lib.ref_shim_linalg.argtypes = [ci, ci, vp, vp, vp]
         lib.ref_chain_restore_random.restype = ci
         lib.ref_chain_restore_random.argtypes = [vp, vp, vp]
     _LIBS[which] = lib
@@ -381,15 +379,24 @@ def ref_dummy_matrices():
     return cov, err
 
 
-def ref_shim_linalg(which, a):
+def shim_linalg(which, a):
     """The shim's TDecompChol (0), TMatrixD::Invert (1) or TMatrixDSymEigen (2) on a square matrix:
-    (matrix, values) as the reference's code receives them."""
-    lib = load("ref")
+    (matrix, values) as the reference's code receives them (oracle/shim_linalg.cc)."""
+    if "shim" not in _LIBS:
+        path = os.path.join(HERE, "_build", "libsmcmc_shim.so")
+        if not os.path.exists(path):
+            build(("orc",))
+        lib = ctypes.CDLL(path)
+        lib.shim_linalg.restype = ctypes.c_int
+        lib.shim_linalg.argtypes = [ctypes.c_int, ctypes.c_int] + [ctypes.c_void_p] * 3
+        lib.shim_last_error.restype = ctypes.c_char_p
+        _LIBS["shim"] = lib
+    lib = _LIBS["shim"]
     a = np.ascontiguousarray(a, dtype=np.float64)
     n = a.shape[0]
     out = np.zeros((n, n))
     values = np.zeros(n)
-    rc = lib.ref_shim_linalg(which, n, _ptr(a), _ptr(out), _ptr(values))
+    rc = lib.shim_linalg(which, n, _ptr(a), _ptr(out), _ptr(values))
     if rc < 0:
-        raise RuntimeError(lib.ref_last_error().decode())
+        raise RuntimeError(lib.shim_last_error().decode())
     return (out, values) if rc == 0 else (None, None)

@@ -1,14 +1,14 @@
 // oracle/ref_driver.cc -- builds oracle/_ref/libsmcmc_ref.so.
 //
 // This translation unit #includes the reference's OWN headers, unmodified,
-// from where they lie under /root/reference (never copied into this repo)
+// from a checkout of the reference project (never copied into this repo)
 // and exposes them through the single-chain C interface of chain_api.h.
 // ROOT is replaced by oracle/rootshim.  The reference's global gRandom is
 // pointed at an injected generator that serves the counter-based stream of
 // include/smcmc_rng.h, so the reference consumes exactly the draws the device
 // consumes.  TEST INFRASTRUCTURE ONLY (see chain_api.h).
 //
-// Build: oracle/Makefile target `ref` (needs /root/reference).
+// Build: oracle/Makefile target `ref` (needs REFERENCE=<reference checkout>).
 
 // Standard and shim headers first, so that the access-specifier override
 // below only touches the reference's own classes.
@@ -584,46 +584,6 @@ int ref_dummy_matrices(double* covariance, double* error) {
     if (error) std::copy(TDummyLogLikelihood::Error.GetMatrixArray(),
                          TDummyLogLikelihood::Error.GetMatrixArray() + 10000, error);
     return 0;
-}
-
-// The ROOT linear algebra the reference calls, as restated in oracle/rootshim (ROOT itself is
-// absent): exposed so that tests/test_oracle.py can hold it against LAPACK (numpy) -- an
-// independent implementation -- on random symmetric positive definite matrices.
-//   which 0: TDecompChol::Decompose -> U (upper, U^T U = a)          TSimpleMCMC.H:1100-1118
-//   which 1: TMatrixD::Invert                                          TSimpleHMC.H:806-812
-//   which 2: TMatrixDSymEigen -> out = eigenvectors in columns, values = eigenvalues descending
-//            (TSimpleMCMC.H:1287-1301, TSimpleHMC.H:786-800)
-int ref_shim_linalg(int which, int n, const double* a, double* out, double* values) {
-    return Guard([&]() {
-        if (which == 2) {
-            TMatrixDSym m(n);
-            for (int i = 0; i < n; ++i)
-                for (int j = 0; j < n; ++j) m(i, j) = a[(size_t)i * n + j];
-            TMatrixDSymEigen eig(m);
-            const TMatrixD& v = eig.GetEigenVectors();
-            const TVectorD& w = eig.GetEigenValues();
-            for (int i = 0; i < n; ++i) {
-                values[i] = w(i);
-                for (int j = 0; j < n; ++j) out[(size_t)i * n + j] = v(i, j);
-            }
-            return 0;
-        }
-        TMatrixD m(n, n);
-        for (int i = 0; i < n; ++i)
-            for (int j = 0; j < n; ++j) m(i, j) = a[(size_t)i * n + j];
-        if (which == 0) {
-            TDecompChol chol(m);
-            if (!chol.Decompose()) return 1;
-            const TMatrixD& u = chol.GetU();
-            for (int i = 0; i < n; ++i)
-                for (int j = 0; j < n; ++j) out[(size_t)i * n + j] = u(i, j);
-            return 0;
-        }
-        m.Invert();
-        for (int i = 0; i < n; ++i)
-            for (int j = 0; j < n; ++j) out[(size_t)i * n + j] = m(i, j);
-        return 0;
-    });
 }
 
 // The reference's own toy-input generators (example/Simulated.H:17-53 and

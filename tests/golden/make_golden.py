@@ -1,12 +1,14 @@
 """Generate the golden vectors under tests/golden/ by running the REFERENCE's
-own code (oracle/_ref/libsmcmc_ref.so = /root/reference headers compiled
+own code (oracle/_ref/libsmcmc_ref.so = the reference's headers compiled
 unmodified against oracle/rootshim) on seeded inputs.
 
-Run in the build container (needs /root/reference):
-    python tests/golden/make_golden.py
+Needs a checkout of the reference:
+    REFERENCE=<checkout> python tests/golden/make_golden.py
 The reference ships no golden vectors of its own (SURVEY.md section 4), so these
 files are how its behaviour is pinned for the machines where the reference
-tree is absent.
+tree is absent.  `python tests/golden/make_golden.py fresh` also runs without
+the reference: fresh_seeds.npz then comes from the oracle port and says so in
+its `source` entry.
 """
 import os
 import sys
@@ -315,9 +317,79 @@ def make_hmc():
     print("hmc.npz: %d arrays" % len(out))
 
 
+# ---------------------------------------------------------------------------
+# Fresh seeds (tests/test_oracle.py::test_port_equals_reference_on_fresh_inputs and
+# ::test_fake2_port_equals_reference_on_fresh_inputs): seeds and points that no other
+# golden file uses.  The full traces are too large to commit, so fresh_seeds.npz holds a
+# SHA-256 of every array (bit-for-bit comparison) and a seeded sample of steps (readable
+# failures).  `source` names the build that produced the file: "reference" when
+# oracle/_ref was built, otherwise "port" (the oracle port, itself pinned to the reference
+# by the other golden files).
+# ---------------------------------------------------------------------------
+FRESH_CHAINS = [(0, 5, 1500), (0, 3, 800), (2, 75, 1200), (3, 100, 800)]
+FRESH_CHAIN_IDS = (1, 9)
+FRESH_SAMPLE_STEPS = 24
+
+
+def digest(a):
+    """SHA-256 of an array's dtype, shape and bytes (NaNs made canonical) as 32 uint8."""
+    import hashlib
+    a = np.ascontiguousarray(a)
+    if a.dtype.kind == "f":
+        a = np.where(np.isnan(a), np.nan, a)
+    h = hashlib.sha256(("%s%s" % (a.dtype.str, a.shape)).encode())
+    h.update(a.tobytes())
+    return np.frombuffer(h.digest(), np.uint8)
+
+
+def fresh_chain(which, kind, dim, n, chain):
+    """(Start() result, trace of n steps) of one fresh-seed chain."""
+    c = cc.CpuChain(which, kind, dim, 77, chain)
+    ok = c.start(np.random.default_rng(chain).uniform(-0.2, 0.2, dim))
+    return ok, c.step(n)
+
+
+def fresh_sample(n, chain):
+    return np.sort(np.random.default_rng(100 + chain).choice(n, FRESH_SAMPLE_STEPS, replace=False))
+
+
+def fresh_fake2(which):
+    """example2's likelihood and histograms at 30 new points on new events, including negative
+    event counts (the penalty branches) and a point where every event is cut."""
+    events, data = synth.fake2_inputs(120, 90, 10, seed=77)
+    c = cc.CpuChain(which, cc.LLH_FAKE2, 9, 1, 0)
+    c.set_fake(events, data, 1.0)
+    rng = np.random.default_rng(5)
+    pts = rng.normal(0, 2, (30, 9))
+    pts[:, 0] = rng.uniform(-60, 400, 30)
+    pts[:, 1] = rng.uniform(-60, 400, 30)
+    pts[0, 2] = 2000.0      # exp overflows: every mass is inf, every event cut
+    return np.array([c.llh(p) for p in pts]), np.array([c.fake_hist(p) for p in pts])
+
+
+def make_fresh():
+    which = "ref" if cc.available("ref") else "orc"
+    out = {"source": np.array("reference" if which == "ref" else "port")}
+    for kind, dim, n in FRESH_CHAINS:
+        for chain in FRESH_CHAIN_IDS:
+            ok, tr = fresh_chain(which, kind, dim, n, chain)
+            p = "k%d_d%d_c%d/" % (kind, dim, chain)
+            out[p + "ok"] = np.array(ok)
+            rows = fresh_sample(n, chain)
+            for k, v in tr.items():
+                out[p + k + "_sha256"] = digest(v)
+                out[p + k + "_sample"] = v[rows]
+    llh, hist = fresh_fake2(which)
+    out["fake2/llh"] = llh
+    out["fake2/hist_sha256"] = digest(hist)
+    out["fake2/hist_sample"] = hist[::7]
+    np.savez_compressed(os.path.join(HERE, "fresh_seeds.npz"), **out)
+    print("fresh_seeds.npz: %d arrays from the %s build" % (len(out), out["source"]))
+
+
 if __name__ == "__main__":
     cc.build()
-    which = sys.argv[1:] or ["fake", "fake2", "chains", "hmc", "vaat"]
+    which = sys.argv[1:] or ["fake", "fake2", "chains", "hmc", "vaat", "fresh"]
     if "vaat" in which:
         make_vaat()
     if "fake" in which:
@@ -328,3 +400,5 @@ if __name__ == "__main__":
         make_chains()
     if "hmc" in which:
         make_hmc()
+    if "fresh" in which:
+        make_fresh()

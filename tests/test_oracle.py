@@ -85,19 +85,26 @@ def test_fake_schedule_matches_golden(checkers, have_ref, which):
 
 
 def test_port_equals_reference_on_fresh_inputs(checkers, have_ref):
-    """Not just the committed vectors: new seeds, every likelihood kind."""
-    if not have_ref:
-        pytest.skip("reference-backed checker not built here")
-    cc = checkers
-    for kind, dim, n in [(0, 5, 1500), (0, 3, 800), (2, 75, 1200), (3, 100, 800)]:
-        for chain in (1, 9):
-            a = cc.CpuChain("ref", kind, dim, 77, chain)
-            b = cc.CpuChain("orc", kind, dim, 77, chain)
-            x0 = np.random.default_rng(chain).uniform(-0.2, 0.2, dim)
-            assert a.start(x0) == b.start(x0)
-            ta, tb = a.step(n), b.step(n)
-            for k in ta:
-                assert np.array_equal(ta[k], tb[k]), (kind, k)
+    """Not just the committed chains: new seeds, every likelihood kind.  The port's traces must
+    match tests/golden/fresh_seeds.npz bit for bit (a SHA-256 per array, a sample of steps for
+    a readable failure; `source` there names the build that made it) and, where the
+    reference-backed checker is built, the reference's own traces."""
+    from golden.make_golden import FRESH_CHAINS, FRESH_CHAIN_IDS, digest, fresh_chain, fresh_sample
+    g = golden("fresh_seeds.npz")
+    for kind, dim, n in FRESH_CHAINS:
+        for chain in FRESH_CHAIN_IDS:
+            p = "k%d_d%d_c%d/" % (kind, dim, chain)
+            ok, tb = fresh_chain("orc", kind, dim, n, chain)
+            assert ok == int(g[p + "ok"])
+            rows = fresh_sample(n, chain)
+            for k in tb:
+                assert np.array_equal(tb[k][rows], g[p + k + "_sample"]), (kind, dim, chain, k)
+                assert np.array_equal(digest(tb[k]), g[p + k + "_sha256"]), (kind, dim, chain, k)
+            if have_ref:
+                ok_ref, ta = fresh_chain("ref", kind, dim, n, chain)
+                assert ok_ref == ok
+                for k in ta:
+                    assert np.array_equal(ta[k], tb[k]), (kind, k)
 
 
 def test_cholesky_identity(checkers):
@@ -339,25 +346,19 @@ def test_fake2_schedule_matches_golden(checkers, have_ref, which):
 
 def test_fake2_port_equals_reference_on_fresh_inputs(checkers, have_ref):
     """New events and points, including negative event counts (the penalty
-    branches) and a point where every event is cut (x / 0 normalisation)."""
-    if not have_ref:
-        pytest.skip("reference-backed checker not built here")
-    from smcmc_b200 import synth
-    events, data = synth.fake2_inputs(120, 90, 10, seed=77)
-    a = checkers.CpuChain("orc", checkers.LLH_FAKE2, 9, 1, 0)
-    b = checkers.CpuChain("ref", checkers.LLH_FAKE2, 9, 1, 0)
-    a.set_fake(events, data, 1.0)
-    b.set_fake(events, data, 1.0)
-    rng = np.random.default_rng(5)
-    pts = rng.normal(0, 2, (30, 9))
-    pts[:, 0] = rng.uniform(-60, 400, 30)
-    pts[:, 1] = rng.uniform(-60, 400, 30)
-    pts[0, 2] = 2000.0      # exp overflows: every mass is inf, every event cut
-    for p in pts:
-        la, lb = a.llh(p), b.llh(p)
-        assert la == lb or (np.isnan(la) and np.isnan(lb))
-        assert np.array_equal(a.fake_hist(p), b.fake_hist(p), equal_nan=True)
-    assert np.isnan(a.llh(pts[0]))
+    branches) and a point where every event is cut (x / 0 normalisation): the port
+    against tests/golden/fresh_seeds.npz and, where it is built, the reference."""
+    from golden.make_golden import digest, fresh_fake2
+    g = golden("fresh_seeds.npz")
+    llh, hist = fresh_fake2("orc")
+    assert np.array_equal(llh, g["fake2/llh"], equal_nan=True)
+    assert np.array_equal(hist[::7], g["fake2/hist_sample"], equal_nan=True)
+    assert np.array_equal(digest(hist), g["fake2/hist_sha256"])
+    if have_ref:
+        llh_ref, hist_ref = fresh_fake2("ref")
+        assert np.array_equal(llh, llh_ref, equal_nan=True)
+        assert np.array_equal(hist, hist_ref, equal_nan=True)
+    assert np.isnan(llh[0])
 
 
 # ---------------------------------------------------------------------------
@@ -396,14 +397,13 @@ def test_vaat_chain_matches_golden(checkers, have_ref, which, name):
 
 
 @pytest.mark.parametrize("n", [2, 5, 50, 100])
-def test_shim_linear_algebra_against_lapack(checkers, have_ref, n):
+def test_shim_linear_algebra_against_lapack(checkers, n):
     """ROOT is absent, so `oracle/_ref` runs the reference's headers on a restatement of the ROOT
-    linear algebra they call (oracle/rootshim: TDecompChol, TMatrixD::Invert, TMatrixDSymEigen).
+    linear algebra they call (oracle/rootshim: TDecompChol, TMatrixD::Invert, TMatrixDSymEigen),
+    here compiled on its own (oracle/shim_linalg.cc).
     Held here against LAPACK (numpy), an independent implementation, on random symmetric positive
     definite matrices of the sizes the golden chains use: the factor, the inverse and the spectrum
     are unique, so agreement to rounding pins what the shim computes, not how."""
-    if not have_ref:
-        pytest.skip("oracle/_ref not built")
     rng = np.random.default_rng(1000 + n)
     for trial in range(4):
         g = rng.normal(size=(n, 2 * n))
@@ -412,13 +412,13 @@ def test_shim_linear_algebra_against_lapack(checkers, have_ref, n):
             d = np.logspace(0, 3, n)
             a = d[:, None] * (0.98 + 0.02 * np.eye(n)) * d[None, :]
         cond = np.linalg.cond(a)
-        u, _ = checkers.ref_shim_linalg(0, a)
+        u, _ = checkers.shim_linalg(0, a)
         assert np.array_equal(np.tril(u, -1), np.zeros((n, n)))
         assert np.allclose(u, np.linalg.cholesky(a).T, rtol=1e-13 * cond, atol=1e-15 * np.abs(a).max())
-        inv, _ = checkers.ref_shim_linalg(1, a)
+        inv, _ = checkers.shim_linalg(1, a)
         ref = np.linalg.inv(a)
         assert np.abs(inv - ref).max() <= 1e-14 * cond * np.abs(ref).max()
-        vec, val = checkers.ref_shim_linalg(2, a)
+        vec, val = checkers.shim_linalg(2, a)
         w, v = np.linalg.eigh(a)
         w, v = w[::-1], v[:, ::-1]                       # the reference relies on DESCENDING eigenvalues
         assert np.all(np.diff(val) <= 0.0)
@@ -432,4 +432,4 @@ def test_shim_linear_algebra_against_lapack(checkers, have_ref, n):
     # a matrix that is not positive definite: Decompose() fails (TSimpleMCMC.H:1100-1118 takes that branch)
     bad = np.eye(n)
     bad[n - 1, n - 1] = -1.0
-    assert checkers.ref_shim_linalg(0, bad)[0] is None
+    assert checkers.shim_linalg(0, bad)[0] is None
