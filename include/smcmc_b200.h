@@ -269,6 +269,12 @@ int smcmc_fake_counts(smcmc_engine* e, const double* x, int m, uint32_t* out);
  * pairs the filter left to FP64, pairs where a filter decision differs from
  * the FP64 decision}.  The last number must be 0. */
 int smcmc_fake_filter_check(smcmc_engine* e, const double* x, int m, uint64_t* out3);
+/* Diagnostic for the pair kernel's tile skip (DESIGN.md section 4.1): for each
+ * warp of 32 consecutive points and each event tile of the candidate mass bands,
+ * applies the kernel's skip rule, and checks every pair of every skipped tile in
+ * FP64.  out3 = {tiles tested, tiles skipped, pairs of skipped tiles that the
+ * FP64 arithmetic counts}.  The last number must be 0. */
+int smcmc_fake_skip_check(smcmc_engine* e, const double* x, int m, uint64_t* out3);
 /* SMCMC_LLH_UNBINNED, the unbinned counterpart of the event likelihood.  The
  * reference has no such functor (its likelihood is binned); this one is DEFINED
  * HERE on top of the reference's per-event corrections, with the same 9

@@ -190,10 +190,12 @@ struct smcmc_engine {
     DeviceBuffer<FilterChain> fakeFilterChains;
     DeviceBuffer<unsigned long long> fakeStats;
     bool exactOnly = false;
+    bool noTileSkip = false;                        // SMCMC_FAKE_NO_SKIP: the pair kernel evaluates every tile
     DeviceBuffer<smcmc_event> fakeIrregular;
     int64_t fakeClassBase[kFakeClasses] = {0, 0, 0, 0};    // padded event index, multiple of kPairTile
     int64_t fakeClassCount[kFakeClasses] = {0, 0, 0, 0};   // events of the class, padding included
     int64_t fakeClassReal[kFakeClasses] = {0, 0, 0, 0};
+    int64_t fakeBandStart[kFakeClasses][kMassBands] = {};  // first event of each mass band in its class
     int64_t fakeIrregularCount = 0;
     int64_t fakeEventCount = -1;
     DeviceBuffer<double> fakeData;
@@ -578,10 +580,12 @@ struct smcmc_engine {
             L.classBase[c] = fakeClassBase[c];
             L.classCount[c] = fakeClassCount[c];
             L.classReal[c] = fakeClassReal[c];
+            for (int b = 0; b < kMassBands; ++b) L.bandStart[c][b] = fakeBandStart[c][b];
             L.chunkBase[c] = chunks;
             chunks += (int)((fakeClassCount[c] + chunkEvents - 1) / chunkEvents);
         }
         L.chunkBase[kFakeClasses] = chunks;
+        L.skipTiles = noTileSkip ? 0 : 1;
         L.chains = fakeChains.get();
         L.filterChains = fakeFilterChains.get();
         L.numPoints = m;
@@ -1135,6 +1139,7 @@ int smcmc_create(const smcmc_config* cfg, smcmc_engine** out) {
         CUDA_CHECK(cudaMemcpy(e->sc.get(), init.data(), sizeof(ChainScalars) * E, cudaMemcpyHostToDevice));
         e->forceGeneric = std::getenv("SMCMC_FAKE_FORCE_GENERIC") != nullptr;
         e->exactOnly = std::getenv("SMCMC_FAKE_EXACT") != nullptr;
+        e->noTileSkip = std::getenv("SMCMC_FAKE_NO_SKIP") != nullptr;
         e->fakeStats.reserve(4);
         CUDA_CHECK(cudaMemset(e->fakeStats.get(), 0, 4 * sizeof(unsigned long long)));
 
@@ -1416,9 +1421,10 @@ int smcmc_fake_set_events(smcmc_engine* e, const smcmc_event* events, int64_t co
         if (count > 0)
             CUDA_CHECK(cub::DeviceRadixSort::SortPairs(nullptr, sortBytes, (unsigned long long*)nullptr,
                                                        (unsigned long long*)nullptr, (unsigned int*)nullptr,
-                                                       (unsigned int*)nullptr, (int)count, 0, 35, e->stream));
+                                                       (unsigned int*)nullptr, (int)count, 0, kSortKeyBits, e->stream));
         auto align = [](size_t b) { return (b + 255) / 256 * 256; };
         const size_t n = (size_t)count;
+        constexpr int kCountSlots = 8 * kBandSlots;            // per (class, mass band), kFakeCountClasses
         const size_t offRaw = 0;
         const size_t offKeysIn = offRaw + align(n * sizeof(smcmc_event));
         const size_t offKeysOut = offKeysIn + align(n * 8);
@@ -1427,18 +1433,18 @@ int smcmc_fake_set_events(smcmc_engine* e, const smcmc_event* events, int64_t co
         const size_t offSort = offIndexOut + align(n * 4);
         const size_t offSmall = offSort + align(sortBytes);
         DeviceBuffer<unsigned char> arena;
-        arena.reserve(offSmall + 512);
+        arena.reserve(offSmall + 1024);
         unsigned char* base0 = arena.get();
         smcmc_event* raw = (smcmc_event*)(base0 + offRaw);
         unsigned long long* keysIn = (unsigned long long*)(base0 + offKeysIn);
         unsigned long long* keysOut = (unsigned long long*)(base0 + offKeysOut);
         unsigned int* indexIn = (unsigned int*)(base0 + offIndexIn);
         unsigned int* indexOut = (unsigned int*)(base0 + offIndexOut);
-        unsigned long long* counters = (unsigned long long*)(base0 + offSmall);        // 16 x u64
-        int64_t* baseDev = (int64_t*)(base0 + offSmall + 128);                           // 8 x i64
-        int64_t* startDev = (int64_t*)(base0 + offSmall + 192);                          // 8 x i64
-        CUDA_CHECK(cudaMemsetAsync(counters, 0, 16 * sizeof(unsigned long long), e->stream));
-        unsigned long long hostCount[8] = {0};
+        unsigned long long* counters = (unsigned long long*)(base0 + offSmall);        // 64 x u64
+        int64_t* baseDev = (int64_t*)(base0 + offSmall + 512);                           // 8 x i64
+        int64_t* startDev = (int64_t*)(base0 + offSmall + 576);                          // 8 x i64
+        CUDA_CHECK(cudaMemsetAsync(counters, 0, kCountSlots * sizeof(unsigned long long), e->stream));
+        unsigned long long bandCount[kCountSlots] = {0};
         if (count > 0) {
             CUDA_CHECK(cudaMemcpyAsync(raw, events, sizeof(smcmc_event) * count, cudaMemcpyHostToDevice, e->stream));
             kFakeCountClasses<<<ceilDiv(count, 256), 256, 0, e->stream>>>(raw, count, counters, e->forceGeneric);
@@ -1447,11 +1453,14 @@ int smcmc_fake_set_events(smcmc_engine* e, const smcmc_event* events, int64_t co
             kFakeSortKeys<<<ceilDiv(count, 256), 256, 0, e->stream>>>(raw, count, keysIn, indexIn, e->forceGeneric);
             e->launched();
             CUDA_CHECK(cub::DeviceRadixSort::SortPairs(base0 + offSort, sortBytes, keysIn, keysOut, indexIn, indexOut,
-                                                       (int)count, 0, 35, e->stream));
+                                                       (int)count, 0, kSortKeyBits, e->stream));
             e->launched();
-            CUDA_CHECK(cudaMemcpyAsync(hostCount, counters, 8 * sizeof(unsigned long long), cudaMemcpyDeviceToHost, e->stream));
+            CUDA_CHECK(cudaMemcpyAsync(bandCount, counters, sizeof(bandCount), cudaMemcpyDeviceToHost, e->stream));
             CUDA_CHECK(cudaStreamSynchronize(e->stream));
         }
+        unsigned long long hostCount[8] = {0};
+        for (int c = 0; c < 8; ++c)
+            for (int b = 0; b < kBandSlots; ++b) hostCount[c] += bandCount[c * kBandSlots + b];
         // class segments are padded to whole tiles of kPairTile events
         int64_t base[8] = {0}, sortedStart[8] = {0};
         int64_t total = 0, seen = 0;
@@ -1459,6 +1468,11 @@ int smcmc_fake_set_events(smcmc_engine* e, const smcmc_event* events, int64_t co
             base[c] = total;
             sortedStart[c] = seen;
             seen += (int64_t)hostCount[c];
+            int64_t inClass = 0;
+            for (int b = 0; b < kMassBands; ++b) {
+                e->fakeBandStart[c][b] = inClass;
+                inClass += (int64_t)bandCount[c * kBandSlots + b];
+            }
             e->fakeClassBase[c] = total;
             e->fakeClassReal[c] = (int64_t)hostCount[c];
             e->fakeClassCount[c] = ((int64_t)hostCount[c] + kPairTile - 1) / kPairTile * kPairTile;
@@ -1624,6 +1638,26 @@ int smcmc_fake_filter_check(smcmc_engine* e, const double* x, int m, uint64_t* o
         CUDA_CHECK(cudaMemsetAsync(e->fakeStats.get(), 0, 4 * sizeof(unsigned long long), e->stream));
         dim3 grid(512, ceilDiv(m, 128));
         kFakeVerifyFilter<<<grid, 128, 0, e->stream>>>(L, e->fakeStats.get());
+        e->launched();
+        unsigned long long host[4];
+        CUDA_CHECK(cudaMemcpyAsync(host, e->fakeStats.get(), sizeof(host), cudaMemcpyDeviceToHost, e->stream));
+        CUDA_CHECK(cudaStreamSynchronize(e->stream));
+        for (int i = 0; i < 3; ++i) out3[i] = host[i];
+    });
+}
+
+int smcmc_fake_skip_check(smcmc_engine* e, const double* x, int m, uint64_t* out3) {
+    return guarded(e, [&]() {
+        if (e->cfg.likelihood != SMCMC_LLH_FAKE && e->cfg.likelihood != SMCMC_LLH_FAKE2)
+            throw Error(SMCMC_ERR_LOGIC, "engine was not created with SMCMC_LLH_FAKE or SMCMC_LLH_FAKE2");
+        if (!out3) throw Error(SMCMC_ERR_INVALID_ARGUMENT, "null output");
+        e->wantFullCounts = true;
+        try { evalHost(e, x, m, nullptr, nullptr); } catch (...) { e->wantFullCounts = false; throw; }   // fills the per-chain constants for these points
+        e->wantFullCounts = false;
+        PairLaunch L = e->pairLaunch(m, e->fakeCountStride);
+        CUDA_CHECK(cudaMemsetAsync(e->fakeStats.get(), 0, 4 * sizeof(unsigned long long), e->stream));
+        dim3 grid(256, ceilDiv(m, 128));
+        kFakeSkipCheck<<<grid, 128, 0, e->stream>>>(L, e->fakeStats.get());
         e->launched();
         unsigned long long host[4];
         CUDA_CHECK(cudaMemcpyAsync(host, e->fakeStats.get(), sizeof(host), cudaMemcpyDeviceToHost, e->stream));

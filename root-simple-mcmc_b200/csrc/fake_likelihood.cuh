@@ -115,28 +115,52 @@ __device__ __forceinline__ int classifyEvent(const smcmc_event& e, PreparedEvent
     return (e.Type == 0 ? 0 : 2) + (e.MuDk > 0 ? 1 : 0);
 }
 
+// Mass bands of the layout: events of a class are grouped by observed Mass around the cut at 500, so
+// that the events above the cut for a whole box of chains fill whole tiles (the tile skip of
+// pairChunk).  Band b holds edge[b-1] <= Mass < edge[b] (massBand); the edges were chosen with
+// scripts/skip_fraction.py.  Bands from kFirstCandidateBand on are the ones whose tiles the pair
+// kernel tests; the layout is only a heuristic, no count depends on it.
+constexpr int kMassBands = 6;
+constexpr int kFirstCandidateBand = 1;
+constexpr int kBandSlots = 8;                // per class in the upload's counters (kFakeCountClasses)
+__device__ __forceinline__ int massBand(double mass) {
+    const double edge[kMassBands - 1] = {450.0, 550.0, 600.0, 700.0, 900.0};
+    int b = 0;
+#pragma unroll
+    for (int k = 0; k < kMassBands - 1; ++k) b += mass >= edge[k] ? 1 : 0;
+    return b;
+}
+__device__ __forceinline__ int eventBand(const smcmc_event& e, int cls) {
+    return cls == kIrregularClass ? 0 : massBand(e.Mass);
+}
+
+// counts[cls * kBandSlots + band]: events per class and mass band.
 __global__ void kFakeCountClasses(const smcmc_event* __restrict__ ev, int64_t n,
-                                  unsigned long long* classCount, int forceGeneric) {
-    __shared__ unsigned int local[8];
-    if (threadIdx.x < 8) local[threadIdx.x] = 0;
+                                  unsigned long long* counts, int forceGeneric) {
+    constexpr int kSlots = 8 * kBandSlots;
+    __shared__ unsigned int local[kSlots];
+    if (threadIdx.x < kSlots) local[threadIdx.x] = 0;
     __syncthreads();
     int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
     if (i < n) {
         PreparedEvent p;
         int cls = forceGeneric ? kIrregularClass : classifyEvent(ev[i], p);
-        atomicAdd(&local[cls], 1u);
+        atomicAdd(&local[cls * kBandSlots + eventBand(ev[i], cls)], 1u);
     }
     __syncthreads();
-    if (threadIdx.x < 8 && local[threadIdx.x])
-        atomicAdd(&classCount[threadIdx.x], (unsigned long long)local[threadIdx.x]);
+    if (threadIdx.x < kSlots && local[threadIdx.x])
+        atomicAdd(&counts[threadIdx.x], (unsigned long long)local[threadIdx.x]);
 }
 
-// Re-layout at upload.  Events are ordered by (class, separation): inside a
-// class the order does not matter for the counts, and ascending separation
-// makes most tiles of the untagged classes lie entirely on one side of every
-// chain's separation cut, so that the pair kernel can skip the per-pair test
-// there (pairChunk).  kFakeSortKeys writes the 64-bit sort keys, the host sorts
-// (key, index) with a device radix sort, kFakeGather fills the class segments.
+// Re-layout at upload.  Events are ordered by (class, mass band, secondary key): inside a class the
+// order does not matter for the counts.  The bands put the events that are above the mass cut for
+// a whole box of chains together (the tile skip).  Inside a band, the untagged classes are ordered
+// by ascending separation, which makes most of their tiles lie entirely on one side of every chain's
+// separation cut, so that the pair kernel can skip the per-pair test there (pairChunk); the tagged
+// classes have no separation test and are ordered by observed mass.  kFakeSortKeys writes the
+// 64-bit sort keys (class << 36 | band << 32 | secondary), the host sorts (key, index) with a device
+// radix sort over bits 0..38, kFakeGather fills the class segments.
+constexpr int kSortKeyBits = 39;
 struct FilterTile;
 __device__ __forceinline__ void storeFilterEvent(FilterTile* tiles, int64_t idx, const PreparedEvent& p);
 
@@ -146,9 +170,10 @@ __global__ void kFakeSortKeys(const smcmc_event* __restrict__ ev, int64_t n, uns
     if (i >= n) return;
     PreparedEvent p;
     const int cls = forceGeneric ? kIrregularClass : classifyEvent(ev[i], p);
-    unsigned int low = 0;
-    if (cls == 0 || cls == 2) low = __float_as_uint(fabsf(__double2float_rn(p.sep)));   // >= 0: bit order = value order
-    keys[i] = ((unsigned long long)cls << 32) | low;
+    unsigned int low = 0;                     // >= 0: bit order = value order
+    if (cls == 0 || cls == 2) low = __float_as_uint(fabsf(__double2float_rn(p.sep)));
+    else if (cls == 1 || cls == 3) low = __float_as_uint(fabsf(__double2float_rn(ev[i].Mass)));
+    keys[i] = ((unsigned long long)cls << 36) | ((unsigned long long)eventBand(ev[i], cls) << 32) | low;
     index[i] = (unsigned int)i;
 }
 
@@ -159,7 +184,7 @@ __global__ void kFakeGather(const smcmc_event* __restrict__ ev, int64_t n, const
                             smcmc_event* irregular) {
     int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
     if (i >= n) return;
-    const int cls = (int)(keys[i] >> 32);
+    const int cls = (int)(keys[i] >> 36);
     const int64_t rank = i - sortedStart[cls];
     const smcmc_event e = ev[index[i]];
     if (cls == kIrregularClass) {
@@ -337,7 +362,8 @@ struct __align__(16) FilterChain {
     float thr[2];    // 100 / separation scale: signal, background
     float thrEps[2]; // error bound of the comparison  sep <> thr
     uint32_t force;  // 1: the filter is not used for this chain (every pair in FP64)
-    float pad_[2];
+    float cutZ;      // log2(500) - scale*log2(e), rounded up: the tile skip's threshold (tileAllCut)
+    float pad_;
 };
 static_assert(sizeof(FilterChain) == 48, "FilterChain is 48 bytes");
 
@@ -408,7 +434,8 @@ __device__ __forceinline__ void storeFilterChain(FilterChain* dst, int c, const 
         f.thr[k] = __double2float_rn(thr);
         f.thrEps[k] = __double2float_ru(8.0 * u * fabs(thr));
     }
-    f.pad_[0] = f.pad_[1] = 0.f;
+    f.cutZ = __double2float_ru(8.965784284662087 - cp.scale * log2e);     // log2(500)
+    f.pad_ = 0.f;
     dst[c] = f;
 }
 
@@ -512,6 +539,8 @@ struct PairLaunch {
     int64_t classBase[kFakeClasses]; // first (padded) event index of each class, a multiple of kPairTile
     int64_t classCount[kFakeClasses];// events of the class INCLUDING the padding of its last tile
     int64_t classReal[kFakeClasses]; // events of the class without the padding
+    int64_t bandStart[kFakeClasses][kMassBands];   // first event of each mass band, relative to classBase
+    int skipTiles;                   // the tile skip is on (off: SMCMC_FAKE_NO_SKIP)
     int chunkBase[kFakeClasses + 1]; // prefix sum of chunks per class
     int chunkEvents;                 // events per work item (multiple of kPairTile, <= kPairChunk)
     const FakeChainParams* chains;
@@ -520,7 +549,7 @@ struct PairLaunch {
     int pointStride;                 // points the count table has room for
     int blockPoints;                 // points per block of the count table (countIndex); == pointStride: one block
     uint32_t* counts;                // [block][kFakeSlots][blockPoints]
-    unsigned long long* stats;       // optional: [0] unsure pairs
+    unsigned long long* stats;       // optional: [0] unsure pairs, [1] pairs in skipped tiles
 };
 
 // Undecided pairs are not evaluated where they are found (one lane in FP64
@@ -538,7 +567,7 @@ struct PairQueue {
     const PreparedEvent* chunkEvents;
     const FakeChainParams* chains;       // of the CTA's first chain
     unsigned countersAddr;
-    unsigned pad_;
+    unsigned skipped;                    // pairs in tiles skipped by the warps (statistics)
     unsigned count[kPairWarps];
     unsigned entry[kPairWarps][kPairQueueCap];   // (event index in chunk) << 8 | chain index in CTA
 };
@@ -703,6 +732,107 @@ __device__ __forceinline__ void tileLoop(const FilterTile* tile, const FilterCha
     }
 }
 
+// ---------------------------------------------------------------------------
+// The tile skip.
+//
+// Events above the mass cut (exactDecide returns -1: bin 50) produce nothing, and whether an event
+// is cut depends on the chain only through scale, width and skewc:
+//   lm = nomLog + width * dLog * exp(logSigma * skewc) + scale,   cut when lm >= gEdges[50] ~ log 500.
+// width > 0, so over a BOX of chains (the min / max of each of the three over the live chains of a
+// warp) the smallest lm of an event is reached at one corner: the least scale, and
+//   dLog >= 0:  the least width and the least logSigma*skewc  (skewc low if logSigma >= 0, else high)
+//   dLog <  0:  the largest width and the largest logSigma*skewc.
+// In the log2 domain of the filter (ls, d, nl2 = the tile's FP32 records, s = skewc*log2(e),
+// w = width*log2(e)) the test of one event at its corner is
+//   x = ls*s;  t = d*ex2(x);  z = fma(t, w, nl2);   cut for the whole box when  z - err >= cutZ,
+// cutZ = log2(500) - scale*log2(e) at the least scale, rounded up (FilterChain::cutZ).
+//
+// Error bound (u = 2^-24; z_real = nl2 + w*d*2^(ls*s) in real numbers at the real corner):
+//   ls, d, nl2, s, w as floats   rel. error <= u each (nl2, s, w: an FP64 product rounded once)
+//                                 -- the box of the FP32 s and w may lie inside the box of the
+//                                 chains' exact values by as much: the same u, counted here
+//   x = ls*s                     rel. error <= 3u (two inputs, one rounding), |x| <= 16 (filter guards)
+//   ex2.approx(x)                rel. error <= 4u + ln2*3u|x| <= (4 + 2.08|x|)u
+//   t = d*ex2                    rel. error <= (6 + 2.08|x|)u
+//   z = fma(t, w, nl2)           abs. error <= |t w|(7 + 2.08|x|)u + |nl2|u + |z|u
+//                                           <= u[41.4|t w| + 2|nl2|] <= u[41.4|t w| + 32]   (|nl2| <= 16)
+// exactDecide computes lm in FP64 in the reference's order ((nom + d*skew) - nom, times width, plus
+// nom, plus scale; exp within 1 ulp): each step rounds at 2^-53 of numbers below |nomLog| + |lm| +
+// |width d skew|, and gEdges[50], the host-exp pre-image of 500, lies within 2^-51 log 500 of log 500.
+// Together (and the rounding of cutZ from FP64) that is below 2^-45 (|t w| + 32) in log2 units:
+// far below one u, covered by the +1 below.  So the kernel skips only when
+//   z >= cutZ + err,  err = kSkipSafety * u * (42 |t| wHi + 33)
+// (wHi >= w; both the slope and the offset rounded up, the sum with an FMA rounding up).  Then
+// z_real >= cutZ_exact at the corner, every chain of the box has lm >= log 500 beyond the FP64
+// rounding, and exactDecide returns -1 for every pair of the tile: skipping it changes no count.
+// A warp with a `force` chain (non-finite or out-of-range constants, SMCMC_FAKE_EXACT) never
+// skips; lanes without a chain take no part in the box.  NaN in z fails the comparison.
+// ---------------------------------------------------------------------------
+constexpr double kSkipSafety = 2.0;
+struct SkipBox {
+    float sLo, sHi, wLo, wHi;   // skewc*log2(e), width*log2(e) over the live chains of the warp
+    float slope, zCut;          // err = slope |t| + (zCut - cutZ): see above
+    bool valid;                 // the warp may skip tiles
+};
+
+// Warp-collective: every lane of the warp calls it.
+__device__ __forceinline__ SkipBox warpSkipBox(const FilterChain& fc, bool live, bool enabled) {
+    const float inf = __int_as_float(0x7f800000);
+    SkipBox b;
+    b.sLo = live ? fc.scl2 : inf;
+    b.sHi = live ? fc.scl2 : -inf;
+    b.wLo = live ? fc.w2 : inf;
+    b.wHi = live ? fc.w2 : -inf;
+    float cut = live ? fc.cutZ : -inf;
+#pragma unroll
+    for (int o = 16; o > 0; o >>= 1) {
+        b.sLo = fminf(b.sLo, __shfl_xor_sync(0xffffffffu, b.sLo, o));
+        b.sHi = fmaxf(b.sHi, __shfl_xor_sync(0xffffffffu, b.sHi, o));
+        b.wLo = fminf(b.wLo, __shfl_xor_sync(0xffffffffu, b.wLo, o));
+        b.wHi = fmaxf(b.wHi, __shfl_xor_sync(0xffffffffu, b.wHi, o));
+        cut = fmaxf(cut, __shfl_xor_sync(0xffffffffu, cut, o));
+    }
+    const double u = 5.9604644775390625e-8;
+    b.slope = __double2float_ru(kSkipSafety * u * 42.0 * (double)b.wHi);
+    b.zCut = __double2float_ru((double)cut + kSkipSafety * u * 33.0);
+    // (fminf / fmaxf drop NaN: a NaN constant sets force, and force turns the skip off)
+    const bool finite = isfinite(b.sLo) && isfinite(b.sHi) && isfinite(b.wLo) && isfinite(b.wHi) &&
+                        isfinite(cut) && b.wLo >= 0.f;
+    b.valid = __all_sync(0xffffffffu, !(live && fc.force)) && enabled && finite && __any_sync(0xffffffffu, live);
+    return b;
+}
+
+__device__ __forceinline__ bool eventCutForBox(float ls, float d, float nl2, const SkipBox& b) {
+    const bool up = d >= 0.f;
+    const float s = (up == (ls >= 0.f)) ? b.sLo : b.sHi;
+    const float w = up ? b.wLo : b.wHi;
+    const float t = __fmul_rn(d, fastEx2(__fmul_rn(ls, s)));
+    const float z = __fmaf_rn(t, w, nl2);
+    return z >= __fmaf_ru(fabsf(t), b.slope, b.zCut);
+}
+
+// Warp-collective: true when every event of the tile is cut for every chain of the box (each lane
+// tests four events).  Padding records (nl2 = +inf) are cut.
+__device__ __forceinline__ bool tileAllCut(const FilterTile* tile, const SkipBox& b, int lane) {
+    const float4 ls = reinterpret_cast<const float4*>(tile->ls)[lane];
+    const float4 d = reinterpret_cast<const float4*>(tile->d)[lane];
+    const float4 nl = reinterpret_cast<const float4*>(tile->nl2)[lane];
+    const bool cut = eventCutForBox(ls.x, d.x, nl.x, b) & eventCutForBox(ls.y, d.y, nl.y, b) &
+                     eventCutForBox(ls.z, d.z, nl.z, b) & eventCutForBox(ls.w, d.w, nl.w, b);
+    return __all_sync(0xffffffffu, cut);
+}
+
+// A tile of an untagged class that straddles a mass-band boundary is not sorted by separation.
+__device__ __forceinline__ bool tileStraddlesBand(const PairLaunch& L, int cls, int64_t tileFirst) {
+    bool straddles = false;
+#pragma unroll
+    for (int b = 1; b < kMassBands; ++b) {
+        const int64_t s = L.bandStart[cls][b];
+        straddles |= s > tileFirst && s < tileFirst + kPairTile;
+    }
+    return straddles;
+}
+
 template <bool TAGGED>
 __device__ __forceinline__ void pairChunk(const PairLaunch& L, int cls, int64_t first, int count,
                                           int pointBase, FilterTile* tiles, uint64_t* bars,
@@ -728,6 +858,7 @@ __device__ __forceinline__ void pairChunk(const PairLaunch& L, int cls, int64_t 
     if (tid == 0) {
         queue->done[0] = queue->done[1] = 0;
         queue->unsure = 0;
+        queue->skipped = 0;
         queue->cls = cls;
         queue->chunkEvents = L.events + classFirst;
         queue->chains = L.chains + pointBase;
@@ -775,6 +906,12 @@ __device__ __forceinline__ void pairChunk(const PairLaunch& L, int cls, int64_t 
 
     const FilterTile* src = L.filterTiles + classFirst / kPairTile;
     const int numTiles = count / kPairTile;
+    // The tile skip: tested on the tiles that hold events of the candidate bands (the tiles before
+    // them are below the cut for any chain near the bulk of the sample, and pay nothing).
+    const SkipBox box = warpSkipBox(fc, live, L.skipTiles != 0);
+    const int64_t candidate = L.bandStart[cls][kFirstCandidateBand] - first;    // events into the chunk
+    const int firstCandidateTile = candidate <= 0 ? 0 : (int)min((int64_t)numTiles, candidate / kPairTile);
+    const unsigned livePairsPerTile = (unsigned)__popc(__ballot_sync(0xffffffffu, live)) * kPairTile;
     // Two tile buffers.  There is no CTA-wide barrier per tile: a warp that has
     // finished a tile says so with an atomic increment of done[buffer], and the
     // warp that makes the count complete refills the buffer with the tile after
@@ -790,16 +927,24 @@ __device__ __forceinline__ void pairChunk(const PairLaunch& L, int cls, int64_t 
         const int buf = t & 1;
         mbarWait(&bars[buf], (uint32_t)(t >> 1) & 1u);
         const FilterTile* tile = &tiles[buf];
-        // Untagged classes: the events are sorted by separation, so most tiles lie
-        // on one side of the cut for every chain of the CTA and the per-pair
-        // separation test (and the load of the separations) is skipped there.
+        // Untagged classes: inside a mass band the events are sorted by separation, so most tiles
+        // lie on one side of the cut for every chain of the CTA and the per-pair separation test
+        // (and the load of the separations) is skipped there.  A tile across a band boundary is
+        // not sorted: it tests every pair.
         int mode = 0;                             // 0: test every pair, 1: all near, 2: all far
         if (TAGGED) mode = 1;
+        else if (tileStraddlesBand(L, cls, first + (int64_t)t * kPairTile)) mode = 0;
         else if (tile->sep[kPairTile - 1] < sepLow) mode = 1;
         else if (tile->sep[0] > sepHigh) mode = 2;
         // a warp without a live chain (ensembles that do not fill the 256-chain tile) only
-        // keeps the buffer protocol going
-        if (warpLive) {
+        // keeps the buffer protocol going; a warp for whose whole box every event of the tile
+        // is cut has nothing to count in it
+        bool skip = false;
+        if (box.valid && t >= firstCandidateTile) {
+            skip = tileAllCut(tile, box, tid & 31);
+            if (skip && L.stats && (tid & 31) == 0) atomicAdd(&queue->skipped, livePairsPerTile);
+        }
+        if (warpLive && !skip) {
             PairRows rows = nearRows;             // (by value: a pointer to one of two structs puts both on the stack)
             if (mode == 2) {
                 rows.mul = nearRows.farMul;
@@ -840,6 +985,7 @@ __device__ __forceinline__ void pairChunk(const PairLaunch& L, int cls, int64_t 
     if (L.stats) {
         __syncthreads();
         if (tid == 0 && queue->unsure) atomicAdd(&L.stats[0], (unsigned long long)queue->unsure);
+        if (tid == 0 && queue->skipped) atomicAdd(&L.stats[1], (unsigned long long)queue->skipped);
     }
 }
 
@@ -1031,6 +1177,44 @@ __global__ void kFakeVerifyFilter(const PairLaunch L, unsigned long long* stats)
     atomicAdd(&stats[0], pairs);
     atomicAdd(&stats[1], unsure);
     atomicAdd(&stats[2], bad);
+}
+
+// Test kernel for the tile skip: for each warp of 32 consecutive points (blockIdx.y * 4 + warp) and
+// each tile of the candidate bands, the pair kernel's skip rule (warpSkipBox, tileAllCut), and for
+// every pair of every skipped tile the FP64 decision, which must be "cut".  stats[0] = tiles
+// tested, [1] = tiles skipped, [2] = pairs of skipped tiles that exactDecide counts (must be zero).
+__global__ void kFakeSkipCheck(const __grid_constant__ PairLaunch L, unsigned long long* stats) {
+    const int lane = threadIdx.x & 31;
+    const int point = (blockIdx.y * (blockDim.x / 32) + (threadIdx.x >> 5)) * 32 + lane;
+    if (__all_sync(0xffffffffu, point >= L.numPoints)) return;
+    const bool live = point < L.numPoints;
+    FilterChain fc = {};
+    FakeChainParams cp = {};
+    if (live) {
+        fc = L.filterChains[point];
+        cp = L.chains[point];
+    }
+    const SkipBox box = warpSkipBox(fc, live, L.skipTiles != 0);
+    if (!box.valid) return;
+    unsigned long long tested = 0, skipped = 0, bad = 0;
+    for (int cls = 0; cls < kFakeClasses; ++cls) {
+        const int64_t firstTile = L.bandStart[cls][kFirstCandidateBand] / kPairTile;
+        const int64_t tiles = L.classCount[cls] / kPairTile;
+        for (int64_t t = firstTile + blockIdx.x; t < tiles; t += gridDim.x) {
+            const FilterTile* tile = L.filterTiles + L.classBase[cls] / kPairTile + t;
+            ++tested;
+            if (!tileAllCut(tile, box, lane)) continue;
+            ++skipped;
+            if (!live) continue;
+            for (int k = 0; k < kPairTile; ++k)
+                if (exactDecide(L.events[L.classBase[cls] + t * kPairTile + k], cp, cls) >= 0) ++bad;
+        }
+    }
+    if (lane == 0) {
+        atomicAdd(&stats[0], tested);
+        atomicAdd(&stats[1], skipped);
+    }
+    if (bad) atomicAdd(&stats[2], bad);
 }
 
 // Straight transcription of the per-event formula for the events the fast

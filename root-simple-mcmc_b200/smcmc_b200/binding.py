@@ -158,6 +158,7 @@ def load_library():
         "smcmc_fake_histograms": (ci, [vp, vp, ci, vp]),
         "smcmc_fake_counts": (ci, [vp, vp, ci, vp]),
         "smcmc_fake_filter_check": (ci, [vp, vp, ci, vp]),
+        "smcmc_fake_skip_check": (ci, [vp, vp, ci, vp]),
         "smcmc_dummy_set_error": (ci, [vp, vp, ci]),
         "smcmc_dummy_set_mode": (ci, [vp, ci]),
         "smcmc_eval": (ci, [vp, vp, ci, vp]),
@@ -202,7 +203,7 @@ EXPORTED_SYMBOLS = [
     "smcmc_prop_reset_correlations", "smcmc_prop_update", "smcmc_prop_reset",
     "smcmc_prop_force_step", "smcmc_prop_set_scan_dimension", "smcmc_prop_set_center", "smcmc_user_set_ops",
     "smcmc_fake_set_events", "smcmc_fake_set_data", "smcmc_unbinned_set_events", "smcmc_fake_histograms",
-    "smcmc_fake_counts", "smcmc_fake_filter_check",
+    "smcmc_fake_counts", "smcmc_fake_filter_check", "smcmc_fake_skip_check",
     "smcmc_dummy_set_error", "smcmc_dummy_set_mode", "smcmc_eval", "smcmc_start", "smcmc_step",
     "smcmc_step_trace", "smcmc_get", "smcmc_save_state", "smcmc_restore_state",
     "smcmc_get_step_index", "smcmc_set_step_index", "smcmc_launch_count",
@@ -393,6 +394,14 @@ class Engine:
         x = np.ascontiguousarray(x, dtype=np.float64).reshape(-1, self.dim)
         out = np.zeros(3, np.uint64)
         self._check(self.lib.smcmc_fake_filter_check(self.h, _ptr(x), x.shape[0], _ptr(out)))
+        return int(out[0]), int(out[1]), int(out[2])
+
+    def fake_skip_check(self, x):
+        """(tiles tested, tiles skipped, pairs of skipped tiles that FP64 counts) of the
+        pair kernel's tile skip, one box per 32 consecutive points."""
+        x = np.ascontiguousarray(x, dtype=np.float64).reshape(-1, self.dim)
+        out = np.zeros(3, np.uint64)
+        self._check(self.lib.smcmc_fake_skip_check(self.h, _ptr(x), x.shape[0], _ptr(out)))
         return int(out[0]), int(out[1]), int(out[2])
 
     def set_dummy_mode(self, mode):
