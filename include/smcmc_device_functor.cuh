@@ -33,6 +33,37 @@
 // (smcmc_user_set_ops, SMCMC_LLH_USER).  No device function pointer crosses a
 // module boundary: libsmcmc_b200.so calls the HOST launch function, which
 // queues the kernel compiled here on the engine's stream.
+//
+// EVENT functors.  A likelihood that is a sum over an event sample (the shape of
+// the reference's example/FakeLikelihood.H) is written as a functor with a nested
+// Event type and three pieces instead of operator():
+//
+//     struct MyEvents {
+//         struct Event { ... };     // trivially copyable, sizeof <= 128, alignof <= 16
+//         struct Chain { ... };     // per-point constants, trivially copyable
+//         __host__ __device__ Chain  Prepare(const double* x, int n) const;
+//         __host__ __device__ double Term(const Chain& c, const Event& ev) const;
+//         // optional (default: return sum)
+//         __host__ __device__ double Finish(const Chain& c, double sum, int64_t events) const;
+//     };
+//     sMCMC::TSimpleMCMC<MyEvents> mcmc;
+//     mcmc.SetEvents(events);       // std::vector<MyEvents::Event>, prepared on the host
+//
+// The value at a point x is Finish(c, S, N) with c = Prepare(x, n) and S the sum of
+// Term(c, e) over the N events in this order: the events are cut into chunks of
+// EventChunk(N) events in upload order; each chunk sum starts at 0.0 and adds its
+// events in order; the chunk sums are added in chunk order, starting at 0.0.  The
+// chunk length depends on N alone, so a point's value does not depend on how many
+// other points are evaluated with it, on the GPU or on the call, and
+// EventLikelihoodHost() restates it on the host.  On the device (kEventPairs) one
+// CTA evaluates 128 points, one per thread, over one chunk: the chunk's events are
+// staged in shared memory, tile by tile, by TMA bulk copies and read by every
+// thread by broadcast.
+//
+// An event functor has no gradient entry: TSimpleHMC<MyEvents> takes finite
+// differences of the likelihood.  A user sample is not split over GPUs: every
+// engine of a chain-sharded run holds the whole sample, and the event groups of
+// smcmc_comm_init do not reduce a user sum.
 #ifndef SMCMC_DEVICE_FUNCTOR_CUH_SEEN
 #define SMCMC_DEVICE_FUNCTOR_CUH_SEEN
 
@@ -46,8 +77,10 @@
 #include <stdexcept>
 #include <string>
 #include <type_traits>
+#include <vector>
 
 #include "TSimpleMCMC.H"
+#include "smcmc_tma.cuh"
 
 namespace smcmc_user {
 
@@ -204,10 +237,243 @@ private:
     F* fDevice;
 };
 
+// ---------------------------------------------------------------------------
+// Event functors
+// ---------------------------------------------------------------------------
+constexpr int kEventTile = 128;          // events per TMA bulk copy
+constexpr int64_t kEventMinChunk = 1024;
+constexpr int64_t kEventMaxChunk = 32768;
+
+template <class F, class = void>
+struct IsEventFunctor : std::false_type {};
+template <class F>
+struct IsEventFunctor<F, decltype((void)sizeof(typename F::Event))> : std::true_type {};
+
+template <class F, class = void>
+struct HasFinish : std::false_type {};
+template <class F>
+struct HasFinish<F, decltype((void)std::declval<const F&>().Finish(std::declval<const typename F::Chain&>(), 0.0,
+                                                                   (int64_t)0))> : std::true_type {};
+
+template <class F>
+struct CheckEventFunctor {
+    typedef typename F::Event Event;
+    typedef typename F::Chain Chain;
+    static_assert(std::is_trivially_copyable<F>::value, "an event functor is copied to the GPU by value: it must be trivially copyable");
+    static_assert(std::is_trivially_copyable<Event>::value, "F::Event is copied to the GPU by bytes: it must be trivially copyable");
+    static_assert(std::is_trivially_copyable<Chain>::value, "F::Chain must be trivially copyable");
+    static_assert(sizeof(Event) <= 128, "sizeof(F::Event) must be at most 128 bytes (a tile of 128 events is staged in shared memory, double buffered)");
+    static_assert(alignof(Event) <= 16, "alignof(F::Event) must be at most 16 bytes");
+    static constexpr bool value = true;
+};
+
+/// Events per chunk of the fixed summation order: about N/256 rounded up to whole
+/// tiles, at least kEventMinChunk and at most kEventMaxChunk.  A function of N only.
+__host__ __device__ inline int64_t EventChunk(int64_t n) {
+    int64_t c = (n + 255) / 256;
+    c = (c + kEventTile - 1) / kEventTile * kEventTile;
+    return c < kEventMinChunk ? kEventMinChunk : (c > kEventMaxChunk ? kEventMaxChunk : c);
+}
+__host__ __device__ inline int64_t EventChunks(int64_t n) {
+    const int64_t c = EventChunk(n);
+    return (n + c - 1) / c;
+}
+
+template <class F>
+__host__ __device__ inline double EventFinish(const F& f, const typename F::Chain& c, double sum, int64_t n, std::true_type) {
+    return f.Finish(c, sum, n);
+}
+template <class F>
+__host__ __device__ inline double EventFinish(const F&, const typename F::Chain&, double sum, int64_t, std::false_type) {
+    return sum;
+}
+
+/// One CTA = 128 points (one per thread) x one chunk of events.  The chunk is
+/// staged tile by tile (kEventTile events, one cp.async.bulk each, double
+/// buffered); every thread reads each event of the tile by broadcast and keeps one
+/// running sum, written to partial[chunk * stride + point].  The event buffer is
+/// padded to whole tiles, so every bulk copy has the same, 16-byte-multiple size.
+template <class F>
+__global__ void __launch_bounds__(kThreads)
+kEventPairs(const F* __restrict__ f, const typename F::Event* __restrict__ events, int64_t n, int chunkEvents,
+            const double* __restrict__ x, int m, int dim, int pointTiles, int stride, double* __restrict__ partial) {
+    typedef typename F::Event Event;
+    constexpr uint32_t kTileBytes = (uint32_t)(kEventTile * sizeof(Event));
+    __shared__ __align__(128) Event tiles[2][kEventTile];
+    __shared__ __align__(8) uint64_t bars[2];
+    const int tid = threadIdx.x;
+    const int chunk = blockIdx.x / pointTiles;
+    const int point = (blockIdx.x - chunk * pointTiles) * kThreads + tid;
+    const int64_t first = (int64_t)chunk * chunkEvents;
+    const int count = (int)min((int64_t)chunkEvents, n - first);
+    const bool live = point < m;
+    typename F::Chain c;
+    if (live) c = f->Prepare(x + (size_t)point * dim, dim);
+
+    if (tid == 0) {
+        smcmc::mbarInit(&bars[0], 1);
+        smcmc::mbarInit(&bars[1], 1);
+        asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
+    }
+    __syncthreads();
+    const Event* src = events + first;
+    const int numTiles = (count + kEventTile - 1) / kEventTile;
+    if (tid == 0) {
+        smcmc::mbarExpectTx(&bars[0], kTileBytes);
+        smcmc::tmaLoad1D(tiles[0], src, kTileBytes, &bars[0]);
+    }
+    double acc = 0.0;
+    for (int t = 0; t < numTiles; ++t) {
+        const int buf = t & 1;
+        if (tid == 0 && t + 1 < numTiles) {
+            smcmc::mbarExpectTx(&bars[buf ^ 1], kTileBytes);
+            smcmc::tmaLoad1D(tiles[buf ^ 1], src + (size_t)(t + 1) * kEventTile, kTileBytes, &bars[buf ^ 1]);
+        }
+        smcmc::mbarWait(&bars[buf], (uint32_t)(t >> 1) & 1u);
+        const int len = min(kEventTile, count - t * kEventTile);
+        if (live) {
+#pragma unroll 2
+            for (int e = 0; e < len; ++e) acc += f->Term(c, tiles[buf][e]);
+        }
+        __syncthreads();
+    }
+    if (live) partial[(size_t)chunk * stride + point] = acc;
+}
+
+/// The chunk sums of each point added in chunk order, then Finish.
+template <class F>
+__global__ void __launch_bounds__(kThreads)
+kEventFinish(const F* __restrict__ f, const double* __restrict__ partial, int chunks, int stride, int64_t n,
+             const double* __restrict__ x, int m, int dim, double* __restrict__ out) {
+    const int p = blockIdx.x * kThreads + threadIdx.x;
+    if (p >= m) return;
+    double s = 0.0;
+    for (int k = 0; k < chunks; ++k) s += partial[(size_t)k * stride + p];
+    out[p] = EventFinish(*f, f->Prepare(x + (size_t)p * dim, dim), s, n, HasFinish<F>());
+}
+
+/// The value of an event functor at one point, on the host, in the order of the
+/// header comment: the reference the device kernels are compared against.
+template <class F>
+double EventLikelihoodHost(const F& f, const typename F::Event* events, int64_t n, const double* x, int dim) {
+    static_assert(CheckEventFunctor<F>::value, "");
+    const typename F::Chain c = f.Prepare(x, dim);
+    const int64_t chunk = EventChunk(n);
+    double s = 0.0;
+    for (int64_t first = 0; first < n; first += chunk) {
+        const int64_t last = first + chunk < n ? first + chunk : n;
+        double part = 0.0;
+        for (int64_t i = first; i < last; ++i) part += f.Term(c, events[i]);
+        s += part;
+    }
+    return EventFinish(f, c, s, n, HasFinish<F>());
+}
+
+/// The device copies of one event functor and its sample, the partial-sum
+/// scratch, and the launch table.  One EventBinding serves one engine (the scratch
+/// is used on that engine's stream).
+template <class F>
+class EventBinding {
+    static_assert(CheckEventFunctor<F>::value, "");
+
+public:
+    typedef typename F::Event Event;
+
+    EventBinding() : fDevice(nullptr), fEvents(nullptr), fCount(-1), fPartial(nullptr), fPartialSize(0) {}
+    ~EventBinding() {
+        if (fDevice) cudaFree(fDevice);
+        if (fEvents) cudaFree(fEvents);
+        if (fPartial) cudaFree(fPartial);
+    }
+    EventBinding(const EventBinding&) = delete;
+    EventBinding& operator=(const EventBinding&) = delete;
+
+    /// Copy the sample to the GPU, padded with zero bytes to whole tiles.  n = 0 is
+    /// an empty sample (sum 0).  Prepare events on the host before this call.
+    void SetEvents(const Event* events, int64_t n) {
+        if (n < 0 || (n > 0 && !events)) throw std::invalid_argument("SetEvents: bad event array");
+        if (fEvents) Check(cudaFree(fEvents));
+        fEvents = nullptr;
+        const size_t padded = (size_t)((n + kEventTile - 1) / kEventTile) * kEventTile;
+        if (padded > 0) {
+            Check(cudaMalloc((void**)&fEvents, padded * sizeof(Event)));
+            Check(cudaMemset(fEvents, 0, padded * sizeof(Event)));
+            Check(cudaMemcpy(fEvents, events, (size_t)n * sizeof(Event), cudaMemcpyHostToDevice));
+        }
+        fCount = n;
+    }
+    bool HasEvents() const { return fCount >= 0; }
+    int64_t GetEventCount() const { return fCount; }
+
+    /// Copy the functor to the GPU (again).
+    void Upload(const F& host) {
+        if (!fDevice) Check(cudaMalloc((void**)&fDevice, sizeof(F)));
+        Check(cudaMemcpy(fDevice, &host, sizeof(F), cudaMemcpyHostToDevice));
+    }
+    /// Upload the functor and register with an engine created with SMCMC_LLH_USER;
+    /// the sample must have been set.
+    void Bind(smcmc_engine* e, const F& host) {
+        if (!HasEvents()) throw std::logic_error("event functor: no event sample set (SetEvents) before Bind");
+        Upload(host);
+        smcmc_user_ops ops;
+        ops.struct_size = sizeof ops;
+        ops.reserved_ = 0;
+        ops.ctx = this;
+        ops.likelihood = &EventBinding::LaunchLikelihood;
+        ops.gradient = nullptr;                       // finite differences of the likelihood
+        const int rc = smcmc_user_set_ops(e, &ops);
+        if (rc != SMCMC_OK) throw std::logic_error(smcmc_last_error(e));
+    }
+    /// Bind with a sample given as raw bytes (a C entry point of a user library):
+    /// itemsize must be sizeof(Event).
+    void Bind(smcmc_engine* e, const F& host, const void* events, int64_t n, size_t itemsize) {
+        if (itemsize != sizeof(Event))
+            throw std::invalid_argument("event item size " + std::to_string(itemsize) + " != sizeof(Event) " +
+                                        std::to_string(sizeof(Event)));
+        SetEvents(static_cast<const Event*>(events), n);
+        Bind(e, host);
+    }
+
+private:
+    static void Check(cudaError_t rc) {
+        if (rc != cudaSuccess) throw std::runtime_error(std::string("CUDA: ") + cudaGetErrorString(rc));
+    }
+    static int LaunchLikelihood(void* ctx, const double* x, int m, int n, double* out, void* stream) {
+        EventBinding* b = static_cast<EventBinding*>(ctx);
+        cudaStream_t s = (cudaStream_t)stream;
+        const int chunks = (int)EventChunks(b->fCount);
+        const int stride = (m + 31) / 32 * 32;
+        const size_t need = (size_t)chunks * stride;
+        if (need > b->fPartialSize) {              // grows only: stream-ordered on the engine's stream
+            if (b->fPartial) {
+                cudaError_t rc = cudaFreeAsync(b->fPartial, s);
+                if (rc != cudaSuccess) return (int)rc;
+                b->fPartial = nullptr;
+                b->fPartialSize = 0;
+            }
+            cudaError_t rc = cudaMallocAsync((void**)&b->fPartial, need * sizeof(double), s);
+            if (rc != cudaSuccess) return (int)rc;
+            b->fPartialSize = need;
+        }
+        const int pointTiles = (m + kThreads - 1) / kThreads;
+        if (chunks > 0)
+            kEventPairs<F><<<(unsigned)chunks * (unsigned)pointTiles, kThreads, 0, s>>>(
+                b->fDevice, b->fEvents, b->fCount, (int)EventChunk(b->fCount), x, m, n, pointTiles, stride, b->fPartial);
+        kEventFinish<F><<<pointTiles, kThreads, 0, s>>>(b->fDevice, b->fPartial, chunks, stride, b->fCount, x, m, n, out);
+        return (int)cudaGetLastError();
+    }
+
+    F* fDevice;
+    Event* fEvents;
+    int64_t fCount;           // -1: no sample set
+    double* fPartial;         // [chunks][stride]
+    size_t fPartialSize;
+};
+
 }  // namespace smcmc_user
 
 // The sampler side: a likelihood class WITHOUT a built-in id (no kDeviceLikelihood
-// member) is a user device functor.
+// member) is a user device functor; one with a nested Event type is an event functor.
 namespace sMCMC {
 namespace detail {
 template <class L, class Enable>
@@ -217,6 +483,33 @@ struct DeviceBinding {
     void Bind(smcmc_engine* e, L& like) { fBinding.Bind(e, like); }
     void Sync(smcmc_engine*, L& like) { fBinding.Upload(like); }
     smcmc_user::Binding<L> fBinding;
+};
+template <class L>
+struct DeviceBinding<L, typename std::enable_if<smcmc_user::IsEventFunctor<L>::value>::type> {
+    typedef typename L::Event Event;
+    static int Kind() { return SMCMC_LLH_USER; }
+    static bool HasGradient() { return false; }
+    void Bind(smcmc_engine* e, L& like) {
+        if (fHavePending) {
+            fBinding.SetEvents(fPending.data(), (int64_t)fPending.size());
+            std::vector<Event>().swap(fPending);
+            fHavePending = false;
+        }
+        fBinding.Bind(e, like);
+    }
+    void Sync(smcmc_engine*, L& like) { fBinding.Upload(like); }
+    // before the engine exists the sample is kept and uploaded by Bind
+    void SetEvents(smcmc_engine* e, const std::vector<Event>& events) {
+        if (e) {
+            fBinding.SetEvents(events.data(), (int64_t)events.size());
+        } else {
+            fPending = events;
+            fHavePending = true;
+        }
+    }
+    std::vector<Event> fPending;
+    bool fHavePending = false;
+    smcmc_user::EventBinding<L> fBinding;
 };
 }  // namespace detail
 }  // namespace sMCMC

@@ -17,7 +17,7 @@
 #pragma once
 #include "proposal.cuh"
 #include "simple_likelihoods.cuh"
-#include "tma.cuh"
+#include "smcmc_tma.cuh"
 
 namespace smcmc {
 

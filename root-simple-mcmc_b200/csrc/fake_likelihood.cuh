@@ -32,7 +32,7 @@
 
 #include "seqsum.h"
 #include "smcmc_b200.h"
-#include "tma.cuh"
+#include "smcmc_tma.cuh"
 
 namespace smcmc {
 

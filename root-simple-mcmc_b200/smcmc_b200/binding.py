@@ -363,6 +363,22 @@ class Engine:
         if fn(self.h) != 0:
             raise SmcmcError(-3, "%s failed: %s" % (symbol, self.lib.smcmc_last_error(self.h).decode()))
 
+    def bind_user_events(self, lib, symbol, events):
+        """SMCMC_LLH_USER with an EVENT functor (include/smcmc_device_functor.cuh):
+        `symbol(engine, events, n, itemsize)` of a user library uploads the sample
+        and registers the functor.  `events` is an array of n records laid out as
+        the functor's Event (a structured dtype, or rows of a plain one); the
+        library rejects an itemsize other than sizeof(Event).  The sample is
+        copied; the array may be dropped afterwards."""
+        ev = np.ascontiguousarray(events)
+        n = ev.shape[0] if ev.ndim else 1
+        itemsize = ev.itemsize * (int(np.prod(ev.shape[1:])) if ev.ndim > 1 else 1)
+        fn = getattr(lib, symbol)
+        fn.restype = ctypes.c_int
+        fn.argtypes = [ctypes.c_void_p, ctypes.c_void_p, ctypes.c_int64, ctypes.c_size_t]
+        if fn(self.h, ev.ctypes.data if n else None, n, itemsize) != 0:
+            raise SmcmcError(-3, "%s failed (itemsize %d, %d events)" % (symbol, itemsize, n))
+
     # -- likelihood inputs ---------------------------------------------------
     def set_fake_events(self, events):
         ev = np.ascontiguousarray(events, dtype=EVENT_DTYPE)
