@@ -1502,6 +1502,7 @@ int smcmc_fake_set_events(smcmc_engine* e, const smcmc_event* events, int64_t co
         }
         CUDA_CHECK(cudaStreamSynchronize(e->stream));          // the arena goes out of scope; host arrays were read
         e->fakeEventCount = count;
+        e->hmc.gradCacheReady = false;                         // the gradients kept belong to the old sample
     });
 }
 
@@ -1546,6 +1547,7 @@ int smcmc_unbinned_set_events(smcmc_engine* e, const smcmc_event* events, int64_
         e->unbClassCount[0] = count - (int64_t)tagged;
         e->unbClassCount[1] = (int64_t)tagged;
         e->unbEventCount = count;
+        e->hmc.gradCacheReady = false;                 // the gradients kept belong to the old sample
     });
 }
 
@@ -1558,6 +1560,7 @@ int smcmc_fake_set_data(smcmc_engine* e, const double* data150, double exposure)
         CUDA_CHECK(cudaStreamSynchronize(e->stream));
         e->fakeExposure = exposure;
         e->fakeDataSet = true;
+        e->hmc.gradCacheReady = false;                 // the gradients kept belong to the old data
     });
 }
 
