@@ -64,6 +64,32 @@
 // differences of the likelihood.  A user sample is not split over GPUs: every
 // engine of a chain-sharded run holds the whole sample, and the event groups of
 // smcmc_comm_init do not reduce a user sum.
+//
+// BINNED event functors.  A likelihood that fills histograms from the sample and
+// compares them with data (a template fit; example/FakeLikelihood.H) is an event
+// functor with a bin count and a bin rule instead of Term:
+//
+//     struct MyBinned {
+//         struct Event { ... };     // as for event functors
+//         struct Chain { ... };     // per-point constants
+//         static constexpr int kBins = 300;                        // 1 <= kBins <= 512
+//         __host__ __device__ Chain  Prepare(const double* x, int n) const;
+//         __host__ __device__ int    Bin(const Chain& c, const Event& ev) const;   // outside [0, kBins): not counted
+//         __host__ __device__ double Finish(const Chain& c, const smcmc_user::BinCounts& counts, int64_t events) const;
+//     };
+//     sMCMC::TSimpleMCMC<MyBinned> mcmc;  mcmc.SetEvents(events);
+//
+// It is recognised by F::kBins together with F::Event.  The value at x is
+// Finish(c, counts, N) with c = Prepare(x, n) and counts[b] (uint32) the number of
+// events with Bin(c, e) == b.  Counts are integers, so they do not depend on how
+// the device splits the sample, and BinnedCountsHost() / BinnedLikelihoodHost()
+// restate them on the host.  Data histograms live in the functor as fixed-size
+// arrays and change as any member does (GetLogLikelihood() before Start(),
+// SyncLikelihood() after).  On the device (kBinnedPairs) one CTA counts 128 points
+// over one chunk of fewer than 65536 events in private 16-bit shared-memory
+// counters and adds them to a global [kBins][points] table; kBinnedFinish applies
+// Finish, one thread per point.  A binned likelihood is piecewise constant: it has
+// no gradient, and TSimpleHMC refuses it at compile time.
 #ifndef SMCMC_DEVICE_FUNCTOR_CUH_SEEN
 #define SMCMC_DEVICE_FUNCTOR_CUH_SEEN
 
@@ -470,10 +496,346 @@ private:
     size_t fPartialSize;
 };
 
+// ---------------------------------------------------------------------------
+// Binned event functors
+// ---------------------------------------------------------------------------
+constexpr int kBinnedMaxBins = 512;
+// Events per chunk of kBinnedPairs: below 65536, so that a 16-bit counter half
+// never carries into its neighbour.
+constexpr int64_t kBinnedMaxChunk = 65536 - kEventTile;
+static_assert(kBinnedMaxChunk < 65536, "a chunk must not overflow a 16-bit counter");
+
+template <class F, class = void>
+struct IsBinnedFunctor : std::false_type {};
+template <class F>
+struct IsBinnedFunctor<F, decltype((void)F::kBins, (void)sizeof(typename F::Event))> : std::true_type {};
+
+/// counts[b] of one point: a column of the [kBins][stride] count table (stride 1
+/// on the host).
+class BinCounts {
+public:
+    __host__ __device__ BinCounts(const uint32_t* first, size_t stride) : fFirst(first), fStride(stride) {}
+    __host__ __device__ uint32_t operator[](int b) const { return fFirst[(size_t)b * fStride]; }
+
+private:
+    const uint32_t* fFirst;
+    size_t fStride;
+};
+
+template <class F>
+struct CheckBinnedFunctor {
+    static_assert(CheckEventFunctor<F>::value, "");
+    static_assert(F::kBins >= 1 && F::kBins <= kBinnedMaxBins,
+                  "F::kBins must be between 1 and 512 (each bin takes 256 bytes of shared-memory counters per CTA)");
+    static_assert(std::is_same<decltype(std::declval<const F&>().Bin(std::declval<const typename F::Chain&>(),
+                                                                     std::declval<const typename F::Event&>())),
+                               int>::value,
+                  "F::Bin(chain, event) must return int");
+    static constexpr bool value = true;
+};
+
+/// Threads per point of kBinnedPairs: the counters take 256 * kBins bytes per CTA,
+/// so fewer CTAs fit an SM as kBins grows; more threads per point keep about 32
+/// warps resident (e.g. 300 bins: two CTAs of 512 threads).
+template <int Bins>
+struct BinnedShape {
+    static constexpr int kThreadsPerPoint = Bins <= 96 ? 1 : Bins <= 192 ? 2 : Bins <= 384 ? 4 : 8;
+    static constexpr int kCtaThreads = kThreads * kThreadsPerPoint;
+};
+
+/// Events per CTA of one kBinnedPairs launch: the grid (chunks x pointTiles) is as
+/// close to a whole number of waves of `slots` resident CTAs as whole tiles allow,
+/// and a chunk holds at most kBinnedMaxChunk events.  Counts do not depend on it.
+inline int64_t BinnedChunk(int64_t n, int64_t pointTiles, int64_t slots) {
+    if (pointTiles < 1) pointTiles = 1;
+    if (slots < 1) slots = 1;
+    const int64_t work = n * pointTiles;
+    int64_t waves = (work + slots * kBinnedMaxChunk - 1) / (slots * kBinnedMaxChunk);
+    if (waves < 1) waves = 1;
+    int64_t c = (work + slots * waves - 1) / (slots * waves);
+    c = (c + kEventTile - 1) / kEventTile * kEventTile;
+    if (c < kEventTile) c = kEventTile;
+    // rounding up the chunk count can spill a few CTAs into one more wave
+    while (c < kBinnedMaxChunk && (n + c - 1) / c * pointTiles > slots * waves) c += kEventTile;
+    return c > kBinnedMaxChunk ? kBinnedMaxChunk : c;
+}
+
+/// The end of a kBinnedPairs chunk: every non-zero 16-bit half of the CTA's
+/// counters (word bin * 64 + (p & 63), point p in half p >> 6) is added to
+/// counts[bin * stride + base + p] with one global reduction.  All threads of the
+/// CTA call it, with their threadIdx.x as tid, after the barrier that ends the
+/// counting.
+template <int Bins>
+__device__ __forceinline__ void FlushBinCounters(const uint32_t* ctr, uint32_t* counts, int stride, int base, int tid) {
+    for (int w = tid; w < Bins * 64; w += BinnedShape<Bins>::kCtaThreads) {
+        const uint32_t v = ctr[w];
+        if (v) {
+            uint32_t* dst = counts + (size_t)(w >> 6) * stride + base + (w & 63);
+            if (v & 0xffffu) atomicAdd(dst, v & 0xffffu);
+            if (v >> 16) atomicAdd(dst + 64, v >> 16);
+        }
+    }
+}
+
+/// One CTA = 128 points x one chunk of events, 128*T threads (T from kBins): thread
+/// t takes point t & 127 and every T-th event of each tile.  Tiles are staged as in
+/// kEventPairs.  Each point's counters are private to the CTA, in shared memory,
+/// 16 bits wide: word bin * 64 + (p & 63) holds point p in half p >> 6, so the 32
+/// lanes of a warp (32 consecutive points) hit 32 different banks whatever bins
+/// they pick.  An event is counted by one shared-memory atomicAdd of 1 or 1 << 16.
+/// At the end of the chunk every non-zero half is added to the global table
+/// counts[bin * stride + point].
+///
+/// The staging loop is kEventPairs' own, not a shared helper: factoring it into
+/// one device function changed kEventPairs' SASS (its instruction schedule).
+template <class F>
+__global__ void __launch_bounds__(BinnedShape<F::kBins>::kCtaThreads)
+kBinnedPairs(const F* __restrict__ f, const typename F::Event* __restrict__ events, int64_t n, int chunkEvents,
+             const double* __restrict__ x, int m, int dim, int pointTiles, int stride, uint32_t* __restrict__ counts) {
+    typedef typename F::Event Event;
+    constexpr int T = BinnedShape<F::kBins>::kThreadsPerPoint;
+    constexpr int kWords = F::kBins * 64;
+    constexpr uint32_t kTileBytes = (uint32_t)(kEventTile * sizeof(Event));
+    extern __shared__ __align__(128) unsigned char smem[];
+    Event (*tiles)[kEventTile] = reinterpret_cast<Event (*)[kEventTile]>(smem);
+    uint32_t* ctr = reinterpret_cast<uint32_t*>(smem + 2 * kTileBytes);
+    __shared__ __align__(8) uint64_t bars[2];
+    const int tid = threadIdx.x;
+    const int lanePoint = tid & (kThreads - 1);
+    const int sub = tid / kThreads;
+    const int chunk = blockIdx.x / pointTiles;
+    const int base = (blockIdx.x - chunk * pointTiles) * kThreads;
+    const int point = base + lanePoint;
+    const int64_t first = (int64_t)chunk * chunkEvents;
+    const int count = (int)min((int64_t)chunkEvents, n - first);
+    const bool live = point < m;
+    const uint32_t one = lanePoint < 64 ? 1u : (1u << 16);
+    uint32_t* mine = ctr + (lanePoint & 63);
+    typename F::Chain c;
+    if (live) c = f->Prepare(x + (size_t)point * dim, dim);
+    for (int w = tid; w < kWords; w += T * kThreads) ctr[w] = 0u;
+
+    if (tid == 0) {
+        smcmc::mbarInit(&bars[0], 1);
+        smcmc::mbarInit(&bars[1], 1);
+        asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
+    }
+    __syncthreads();
+    const Event* src = events + first;
+    const int numTiles = (count + kEventTile - 1) / kEventTile;
+    if (tid == 0) {
+        smcmc::mbarExpectTx(&bars[0], kTileBytes);
+        smcmc::tmaLoad1D(tiles[0], src, kTileBytes, &bars[0]);
+    }
+    for (int t = 0; t < numTiles; ++t) {
+        const int buf = t & 1;
+        if (tid == 0 && t + 1 < numTiles) {
+            smcmc::mbarExpectTx(&bars[buf ^ 1], kTileBytes);
+            smcmc::tmaLoad1D(tiles[buf ^ 1], src + (size_t)(t + 1) * kEventTile, kTileBytes, &bars[buf ^ 1]);
+        }
+        smcmc::mbarWait(&bars[buf], (uint32_t)(t >> 1) & 1u);
+        const int len = min(kEventTile, count - t * kEventTile);
+        if (live) {
+#pragma unroll 2
+            for (int e = sub; e < len; e += T) {
+                const int b = f->Bin(c, tiles[buf][e]);
+                if ((unsigned)b < (unsigned)F::kBins) atomicAdd(mine + b * 64, one);
+            }
+        }
+        __syncthreads();
+    }
+    FlushBinCounters<F::kBins>(ctr, counts, stride, base, tid);
+}
+
+/// One thread per point: Finish over the point's column of the count table.
+template <class F>
+__global__ void __launch_bounds__(kThreads)
+kBinnedFinish(const F* __restrict__ f, const uint32_t* __restrict__ counts, int stride, int64_t n,
+              const double* __restrict__ x, int m, int dim, double* __restrict__ out) {
+    const int p = blockIdx.x * kThreads + threadIdx.x;
+    if (p >= m) return;
+    out[p] = f->Finish(f->Prepare(x + (size_t)p * dim, dim), BinCounts(counts + p, (size_t)stride), n);
+}
+
+/// counts[b] = the number of the n events with Bin(Prepare(x), e) == b, on the host.
+template <class F>
+void BinnedCountsHost(const F& f, const typename F::Event* events, int64_t n, const double* x, int dim,
+                      uint32_t* counts) {
+    static_assert(CheckBinnedFunctor<F>::value, "");
+    const typename F::Chain c = f.Prepare(x, dim);
+    for (int b = 0; b < F::kBins; ++b) counts[b] = 0;
+    for (int64_t i = 0; i < n; ++i) {
+        const int b = f.Bin(c, events[i]);
+        if ((unsigned)b < (unsigned)F::kBins) ++counts[b];
+    }
+}
+
+/// The value of a binned functor at one point, on the host: Finish(c, counts, n).
+/// Counts are integers, so the device value equals it whenever Prepare and Finish
+/// round alike on the host and the device.
+template <class F>
+double BinnedLikelihoodHost(const F& f, const typename F::Event* events, int64_t n, const double* x, int dim) {
+    std::vector<uint32_t> counts(F::kBins);
+    BinnedCountsHost(f, events, n, x, dim, counts.data());
+    return f.Finish(f.Prepare(x, dim), BinCounts(counts.data(), 1), n);
+}
+
+/// The device copies of one binned functor and its sample, the count table, and
+/// the launch table.  One BinnedBinding serves one engine (the table is used on
+/// that engine's stream).
+template <class F>
+class BinnedBinding {
+    static_assert(CheckBinnedFunctor<F>::value, "");
+
+public:
+    typedef typename F::Event Event;
+    static constexpr int kCtaThreads = BinnedShape<F::kBins>::kCtaThreads;
+    static constexpr size_t kSmemBytes = 2 * kEventTile * sizeof(Event) + (size_t)F::kBins * 64 * sizeof(uint32_t);
+
+    BinnedBinding() : fDevice(nullptr), fEvents(nullptr), fCount(-1), fCounts(nullptr), fCountsSize(0), fSlots(0) {}
+    ~BinnedBinding() {
+        if (fDevice) cudaFree(fDevice);
+        if (fEvents) cudaFree(fEvents);
+        if (fCounts) cudaFree(fCounts);
+    }
+    BinnedBinding(const BinnedBinding&) = delete;
+    BinnedBinding& operator=(const BinnedBinding&) = delete;
+
+    /// Copy the sample to the GPU, padded with zero bytes to whole tiles (the
+    /// padding is never binned).  n = 0 is an empty sample (all counts 0).
+    void SetEvents(const Event* events, int64_t n) {
+        if (n < 0 || (n > 0 && !events)) throw std::invalid_argument("SetEvents: bad event array");
+        if (fEvents) Check(cudaFree(fEvents));
+        fEvents = nullptr;
+        const size_t padded = (size_t)((n + kEventTile - 1) / kEventTile) * kEventTile;
+        if (padded > 0) {
+            Check(cudaMalloc((void**)&fEvents, padded * sizeof(Event)));
+            Check(cudaMemset(fEvents, 0, padded * sizeof(Event)));
+            Check(cudaMemcpy(fEvents, events, (size_t)n * sizeof(Event), cudaMemcpyHostToDevice));
+        }
+        fCount = n;
+    }
+    bool HasEvents() const { return fCount >= 0; }
+    int64_t GetEventCount() const { return fCount; }
+
+    /// Copy the functor to the GPU (again).
+    void Upload(const F& host) {
+        if (!fDevice) Check(cudaMalloc((void**)&fDevice, sizeof(F)));
+        Check(cudaMemcpy(fDevice, &host, sizeof(F), cudaMemcpyHostToDevice));
+    }
+    /// Upload the functor and register with an engine created with SMCMC_LLH_USER;
+    /// the sample must have been set.
+    void Bind(smcmc_engine* e, const F& host) {
+        if (!HasEvents()) throw std::logic_error("binned functor: no event sample set (SetEvents) before Bind");
+        Upload(host);
+        smcmc_user_ops ops;
+        ops.struct_size = sizeof ops;
+        ops.reserved_ = 0;
+        ops.ctx = this;
+        ops.likelihood = &BinnedBinding::LaunchLikelihood;
+        ops.gradient = nullptr;                       // a binned likelihood is piecewise constant
+        const int rc = smcmc_user_set_ops(e, &ops);
+        if (rc != SMCMC_OK) throw std::logic_error(smcmc_last_error(e));
+    }
+    /// Bind with a sample given as raw bytes (a C entry point of a user library):
+    /// itemsize must be sizeof(Event).
+    void Bind(smcmc_engine* e, const F& host, const void* events, int64_t n, size_t itemsize) {
+        if (itemsize != sizeof(Event))
+            throw std::invalid_argument("event item size " + std::to_string(itemsize) + " != sizeof(Event) " +
+                                        std::to_string(sizeof(Event)));
+        SetEvents(static_cast<const Event*>(events), n);
+        Bind(e, host);
+    }
+
+    /// The counts of the functor last uploaded at m host points x[m][dim]:
+    /// out[p * kBins + b], synchronously (the posterior-predictive histogram).
+    void Counts(const double* x, int m, int dim, uint32_t* out) {
+        if (!HasEvents() || !fDevice) throw std::logic_error("binned functor: Counts before SetEvents and Upload");
+        if (m < 1 || dim < 1 || !x || !out) throw std::invalid_argument("Counts: bad point array");
+        const int stride = (m + 31) / 32 * 32;
+        double* dx = nullptr;
+        uint32_t* dc = nullptr;
+        std::vector<uint32_t> table((size_t)F::kBins * stride);
+        cudaError_t rc = cudaMalloc((void**)&dx, (size_t)m * dim * sizeof(double));
+        if (rc == cudaSuccess) rc = cudaMalloc((void**)&dc, table.size() * sizeof(uint32_t));
+        if (rc == cudaSuccess) rc = cudaMemcpy(dx, x, (size_t)m * dim * sizeof(double), cudaMemcpyHostToDevice);
+        if (rc == cudaSuccess) rc = (cudaError_t)Count(dx, m, dim, dc, stride, 0);
+        if (rc == cudaSuccess) rc = cudaMemcpy(table.data(), dc, table.size() * sizeof(uint32_t), cudaMemcpyDeviceToHost);
+        if (dx) cudaFree(dx);
+        if (dc) cudaFree(dc);
+        Check(rc);
+        for (int p = 0; p < m; ++p)
+            for (int b = 0; b < F::kBins; ++b) out[(size_t)p * F::kBins + b] = table[(size_t)b * stride + p];
+    }
+    /// Resident CTAs of kBinnedPairs per SM (queried at the first launch; 0 before it).
+    int ResidentCtas() const { return fResident; }
+
+private:
+    static void Check(cudaError_t rc) {
+        if (rc != cudaSuccess) throw std::runtime_error(std::string("CUDA: ") + cudaGetErrorString(rc));
+    }
+    // clear counts[kBins][stride] and count the sample at m device points, on stream s
+    int Count(const double* x, int m, int dim, uint32_t* counts, int stride, cudaStream_t s) {
+        cudaError_t rc = cudaMemsetAsync(counts, 0, (size_t)F::kBins * stride * sizeof(uint32_t), s);
+        if (rc != cudaSuccess || fCount == 0) return (int)rc;
+        if (fSlots == 0) {                            // kBinnedPairs' occupancy, once
+            int dev = 0, sms = 0;
+            if ((rc = cudaGetDevice(&dev)) != cudaSuccess) return (int)rc;
+            if ((rc = cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev)) != cudaSuccess) return (int)rc;
+            if ((rc = cudaFuncSetAttribute(kBinnedPairs<F>, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                                           (int)kSmemBytes)) != cudaSuccess)
+                return (int)rc;
+            if ((rc = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&fResident, kBinnedPairs<F>, kCtaThreads,
+                                                                    kSmemBytes)) != cudaSuccess)
+                return (int)rc;
+            if (fResident < 1) return (int)cudaErrorInvalidConfiguration;
+            fSlots = (int64_t)sms * fResident;
+        }
+        const int pointTiles = (m + kThreads - 1) / kThreads;
+        const int64_t chunk = BinnedChunk(fCount, pointTiles, fSlots);
+        if (chunk >= 65536) return (int)cudaErrorInvalidValue;   // a 16-bit counter would overflow
+        const int64_t chunks = (fCount + chunk - 1) / chunk;
+        kBinnedPairs<F><<<(unsigned)(chunks * pointTiles), kCtaThreads, kSmemBytes, s>>>(
+            fDevice, fEvents, fCount, (int)chunk, x, m, dim, pointTiles, stride, counts);
+        return (int)cudaGetLastError();
+    }
+    static int LaunchLikelihood(void* ctx, const double* x, int m, int n, double* out, void* stream) {
+        BinnedBinding* b = static_cast<BinnedBinding*>(ctx);
+        cudaStream_t s = (cudaStream_t)stream;
+        const int stride = (m + 31) / 32 * 32;
+        const size_t need = (size_t)F::kBins * stride;
+        if (need > b->fCountsSize) {                  // grows only: stream-ordered on the engine's stream
+            if (b->fCounts) {
+                cudaError_t rc = cudaFreeAsync(b->fCounts, s);
+                if (rc != cudaSuccess) return (int)rc;
+                b->fCounts = nullptr;
+                b->fCountsSize = 0;
+            }
+            cudaError_t rc = cudaMallocAsync((void**)&b->fCounts, need * sizeof(uint32_t), s);
+            if (rc != cudaSuccess) return (int)rc;
+            b->fCountsSize = need;
+        }
+        const int rc = b->Count(x, m, n, b->fCounts, stride, s);
+        if (rc != (int)cudaSuccess) return rc;
+        kBinnedFinish<F><<<(m + kThreads - 1) / kThreads, kThreads, 0, s>>>(b->fDevice, b->fCounts, stride, b->fCount,
+                                                                           x, m, n, out);
+        return (int)cudaGetLastError();
+    }
+
+    F* fDevice;
+    Event* fEvents;
+    int64_t fCount;           // -1: no sample set
+    uint32_t* fCounts;        // [kBins][stride]
+    size_t fCountsSize;
+    int64_t fSlots;           // SMs x resident CTAs of kBinnedPairs; 0 until the first launch
+    int fResident = 0;
+};
+
 }  // namespace smcmc_user
 
 // The sampler side: a likelihood class WITHOUT a built-in id (no kDeviceLikelihood
-// member) is a user device functor; one with a nested Event type is an event functor.
+// member) is a user device functor; one with a nested Event type is an event functor,
+// binned when it also has kBins.
 namespace sMCMC {
 namespace detail {
 template <class L, class Enable>
@@ -484,8 +846,8 @@ struct DeviceBinding {
     void Sync(smcmc_engine*, L& like) { fBinding.Upload(like); }
     smcmc_user::Binding<L> fBinding;
 };
-template <class L>
-struct DeviceBinding<L, typename std::enable_if<smcmc_user::IsEventFunctor<L>::value>::type> {
+template <class L, class B>
+struct EventSampleBinding {
     typedef typename L::Event Event;
     static int Kind() { return SMCMC_LLH_USER; }
     static bool HasGradient() { return false; }
@@ -509,7 +871,17 @@ struct DeviceBinding<L, typename std::enable_if<smcmc_user::IsEventFunctor<L>::v
     }
     std::vector<Event> fPending;
     bool fHavePending = false;
-    smcmc_user::EventBinding<L> fBinding;
+    B fBinding;
+};
+template <class L>
+struct DeviceBinding<L, typename std::enable_if<smcmc_user::IsEventFunctor<L>::value &&
+                                                !smcmc_user::IsBinnedFunctor<L>::value>::type>
+    : EventSampleBinding<L, smcmc_user::EventBinding<L> > {};
+// a binned likelihood is piecewise constant: TSimpleHMC refuses it (kHmcUsable)
+template <class L>
+struct DeviceBinding<L, typename std::enable_if<smcmc_user::IsBinnedFunctor<L>::value>::type>
+    : EventSampleBinding<L, smcmc_user::BinnedBinding<L> > {
+    static constexpr bool kHmcUsable = false;
 };
 }  // namespace detail
 }  // namespace sMCMC
