@@ -90,6 +90,32 @@
 // counters and adds them to a global [kBins][points] table; kBinnedFinish applies
 // Finish, one thread per point.  A binned likelihood is piecewise constant: it has
 // no gradient, and TSimpleHMC refuses it at compile time.
+//
+// WEIGHTED binned event functors.  A histogram filled with a weight per event and
+// per point (Fill(x, w): MC weights, reweighting for systematics) is a binned
+// functor with a Weight, and a Finish that receives the weighted sums:
+//
+//     struct MyWeighted {
+//         struct Event { ... };  struct Chain { ... };
+//         static constexpr int kBins = 150;                        // 1 <= kBins <= 256
+//         __host__ __device__ Chain  Prepare(const double* x, int n) const;
+//         __host__ __device__ int    Bin(const Chain& c, const Event& ev) const;      // outside [0, kBins): cut
+//         __host__ __device__ double Weight(const Chain& c, const Event& ev) const;   // called for events not cut
+//         __host__ __device__ double Finish(const Chain& c, const smcmc_user::BinSums& sums, int64_t events) const;
+//     };
+//
+// It is recognised by F::kBins, F::Event and F::Weight.  The value at x is
+// Finish(c, sums, N) with sums[b] the sum of Weight(c, e) over the events with
+// Bin(c, e) == b, in this order: the events are cut into chunks of
+// WeightedChunk(N) events in upload order; within a chunk each bin's sum starts at
+// 0.0 and adds weights in event order; the chunk sums of a bin are added in chunk
+// order, starting at 0.0.  So, as for event functors, a point's value does not
+// depend on the other points of the call, and WeightedSumsHost() /
+// WeightedBinnedLikelihoodHost() restate it on the host.  The weight of a cut
+// event is never computed, so a NaN or inf it would have reaches no sum.  On the
+// device (kWeightedPairs) each thread keeps one point's FP64 histogram in shared
+// memory over one chunk; kWeightedFinish adds the chunks and applies Finish.
+// TSimpleHMC refuses it, as it refuses a binned functor.
 #ifndef SMCMC_DEVICE_FUNCTOR_CUH_SEEN
 #define SMCMC_DEVICE_FUNCTOR_CUH_SEEN
 
@@ -395,28 +421,22 @@ double EventLikelihoodHost(const F& f, const typename F::Event* events, int64_t 
     return EventFinish(f, c, s, n, HasFinish<F>());
 }
 
-/// The device copies of one event functor and its sample, the partial-sum
-/// scratch, and the launch table.  One EventBinding serves one engine (the scratch
-/// is used on that engine's stream).
-template <class F>
-class EventBinding {
-    static_assert(CheckEventFunctor<F>::value, "");
-
+/// The device copy of an event sample, padded with zero bytes to whole tiles so
+/// that every bulk copy of the staging loops has the same, 16-byte-multiple size
+/// (the padding is never evaluated).  Shared by the event, binned and weighted
+/// bindings.
+template <class Event>
+class EventSample {
 public:
-    typedef typename F::Event Event;
-
-    EventBinding() : fDevice(nullptr), fEvents(nullptr), fCount(-1), fPartial(nullptr), fPartialSize(0) {}
-    ~EventBinding() {
-        if (fDevice) cudaFree(fDevice);
+    EventSample() : fEvents(nullptr), fCount(-1) {}
+    ~EventSample() {
         if (fEvents) cudaFree(fEvents);
-        if (fPartial) cudaFree(fPartial);
     }
-    EventBinding(const EventBinding&) = delete;
-    EventBinding& operator=(const EventBinding&) = delete;
+    EventSample(const EventSample&) = delete;
+    EventSample& operator=(const EventSample&) = delete;
 
-    /// Copy the sample to the GPU, padded with zero bytes to whole tiles.  n = 0 is
-    /// an empty sample (sum 0).  Prepare events on the host before this call.
-    void SetEvents(const Event* events, int64_t n) {
+    /// Copy n events to the GPU.  n = 0 is an empty sample.
+    void Set(const Event* events, int64_t n) {
         if (n < 0 || (n > 0 && !events)) throw std::invalid_argument("SetEvents: bad event array");
         if (fEvents) Check(cudaFree(fEvents));
         fEvents = nullptr;
@@ -428,8 +448,41 @@ public:
         }
         fCount = n;
     }
-    bool HasEvents() const { return fCount >= 0; }
-    int64_t GetEventCount() const { return fCount; }
+    bool Has() const { return fCount >= 0; }
+    int64_t Count() const { return fCount; }       // -1: no sample set
+    const Event* Data() const { return fEvents; }
+
+private:
+    static void Check(cudaError_t rc) {
+        if (rc != cudaSuccess) throw std::runtime_error(std::string("CUDA: ") + cudaGetErrorString(rc));
+    }
+    Event* fEvents;
+    int64_t fCount;
+};
+
+/// The device copies of one event functor and its sample, the partial-sum
+/// scratch, and the launch table.  One EventBinding serves one engine (the scratch
+/// is used on that engine's stream).
+template <class F>
+class EventBinding {
+    static_assert(CheckEventFunctor<F>::value, "");
+
+public:
+    typedef typename F::Event Event;
+
+    EventBinding() : fDevice(nullptr), fPartial(nullptr), fPartialSize(0) {}
+    ~EventBinding() {
+        if (fDevice) cudaFree(fDevice);
+        if (fPartial) cudaFree(fPartial);
+    }
+    EventBinding(const EventBinding&) = delete;
+    EventBinding& operator=(const EventBinding&) = delete;
+
+    /// Copy the sample to the GPU.  n = 0 is an empty sample (sum 0).  Prepare
+    /// events on the host before this call.
+    void SetEvents(const Event* events, int64_t n) { fSample.Set(events, n); }
+    bool HasEvents() const { return fSample.Has(); }
+    int64_t GetEventCount() const { return fSample.Count(); }
 
     /// Copy the functor to the GPU (again).
     void Upload(const F& host) {
@@ -467,7 +520,8 @@ private:
     static int LaunchLikelihood(void* ctx, const double* x, int m, int n, double* out, void* stream) {
         EventBinding* b = static_cast<EventBinding*>(ctx);
         cudaStream_t s = (cudaStream_t)stream;
-        const int chunks = (int)EventChunks(b->fCount);
+        const int64_t count = b->fSample.Count();
+        const int chunks = (int)EventChunks(count);
         const int stride = (m + 31) / 32 * 32;
         const size_t need = (size_t)chunks * stride;
         if (need > b->fPartialSize) {              // grows only: stream-ordered on the engine's stream
@@ -484,14 +538,13 @@ private:
         const int pointTiles = (m + kThreads - 1) / kThreads;
         if (chunks > 0)
             kEventPairs<F><<<(unsigned)chunks * (unsigned)pointTiles, kThreads, 0, s>>>(
-                b->fDevice, b->fEvents, b->fCount, (int)EventChunk(b->fCount), x, m, n, pointTiles, stride, b->fPartial);
-        kEventFinish<F><<<pointTiles, kThreads, 0, s>>>(b->fDevice, b->fPartial, chunks, stride, b->fCount, x, m, n, out);
+                b->fDevice, b->fSample.Data(), count, (int)EventChunk(count), x, m, n, pointTiles, stride, b->fPartial);
+        kEventFinish<F><<<pointTiles, kThreads, 0, s>>>(b->fDevice, b->fPartial, chunks, stride, count, x, m, n, out);
         return (int)cudaGetLastError();
     }
 
     F* fDevice;
-    Event* fEvents;
-    int64_t fCount;           // -1: no sample set
+    EventSample<Event> fSample;
     double* fPartial;         // [chunks][stride]
     size_t fPartialSize;
 };
@@ -692,31 +745,18 @@ public:
     static constexpr int kCtaThreads = BinnedShape<F::kBins>::kCtaThreads;
     static constexpr size_t kSmemBytes = 2 * kEventTile * sizeof(Event) + (size_t)F::kBins * 64 * sizeof(uint32_t);
 
-    BinnedBinding() : fDevice(nullptr), fEvents(nullptr), fCount(-1), fCounts(nullptr), fCountsSize(0), fSlots(0) {}
+    BinnedBinding() : fDevice(nullptr), fCounts(nullptr), fCountsSize(0), fSlots(0) {}
     ~BinnedBinding() {
         if (fDevice) cudaFree(fDevice);
-        if (fEvents) cudaFree(fEvents);
         if (fCounts) cudaFree(fCounts);
     }
     BinnedBinding(const BinnedBinding&) = delete;
     BinnedBinding& operator=(const BinnedBinding&) = delete;
 
-    /// Copy the sample to the GPU, padded with zero bytes to whole tiles (the
-    /// padding is never binned).  n = 0 is an empty sample (all counts 0).
-    void SetEvents(const Event* events, int64_t n) {
-        if (n < 0 || (n > 0 && !events)) throw std::invalid_argument("SetEvents: bad event array");
-        if (fEvents) Check(cudaFree(fEvents));
-        fEvents = nullptr;
-        const size_t padded = (size_t)((n + kEventTile - 1) / kEventTile) * kEventTile;
-        if (padded > 0) {
-            Check(cudaMalloc((void**)&fEvents, padded * sizeof(Event)));
-            Check(cudaMemset(fEvents, 0, padded * sizeof(Event)));
-            Check(cudaMemcpy(fEvents, events, (size_t)n * sizeof(Event), cudaMemcpyHostToDevice));
-        }
-        fCount = n;
-    }
-    bool HasEvents() const { return fCount >= 0; }
-    int64_t GetEventCount() const { return fCount; }
+    /// Copy the sample to the GPU.  n = 0 is an empty sample (all counts 0).
+    void SetEvents(const Event* events, int64_t n) { fSample.Set(events, n); }
+    bool HasEvents() const { return fSample.Has(); }
+    int64_t GetEventCount() const { return fSample.Count(); }
 
     /// Copy the functor to the GPU (again).
     void Upload(const F& host) {
@@ -776,8 +816,9 @@ private:
     }
     // clear counts[kBins][stride] and count the sample at m device points, on stream s
     int Count(const double* x, int m, int dim, uint32_t* counts, int stride, cudaStream_t s) {
+        const int64_t count = fSample.Count();
         cudaError_t rc = cudaMemsetAsync(counts, 0, (size_t)F::kBins * stride * sizeof(uint32_t), s);
-        if (rc != cudaSuccess || fCount == 0) return (int)rc;
+        if (rc != cudaSuccess || count == 0) return (int)rc;
         if (fSlots == 0) {                            // kBinnedPairs' occupancy, once
             int dev = 0, sms = 0;
             if ((rc = cudaGetDevice(&dev)) != cudaSuccess) return (int)rc;
@@ -792,11 +833,11 @@ private:
             fSlots = (int64_t)sms * fResident;
         }
         const int pointTiles = (m + kThreads - 1) / kThreads;
-        const int64_t chunk = BinnedChunk(fCount, pointTiles, fSlots);
+        const int64_t chunk = BinnedChunk(count, pointTiles, fSlots);
         if (chunk >= 65536) return (int)cudaErrorInvalidValue;   // a 16-bit counter would overflow
-        const int64_t chunks = (fCount + chunk - 1) / chunk;
+        const int64_t chunks = (count + chunk - 1) / chunk;
         kBinnedPairs<F><<<(unsigned)(chunks * pointTiles), kCtaThreads, kSmemBytes, s>>>(
-            fDevice, fEvents, fCount, (int)chunk, x, m, dim, pointTiles, stride, counts);
+            fDevice, fSample.Data(), count, (int)chunk, x, m, dim, pointTiles, stride, counts);
         return (int)cudaGetLastError();
     }
     static int LaunchLikelihood(void* ctx, const double* x, int m, int n, double* out, void* stream) {
@@ -817,25 +858,333 @@ private:
         }
         const int rc = b->Count(x, m, n, b->fCounts, stride, s);
         if (rc != (int)cudaSuccess) return rc;
-        kBinnedFinish<F><<<(m + kThreads - 1) / kThreads, kThreads, 0, s>>>(b->fDevice, b->fCounts, stride, b->fCount,
-                                                                           x, m, n, out);
+        kBinnedFinish<F><<<(m + kThreads - 1) / kThreads, kThreads, 0, s>>>(b->fDevice, b->fCounts, stride,
+                                                                           b->fSample.Count(), x, m, n, out);
         return (int)cudaGetLastError();
     }
 
     F* fDevice;
-    Event* fEvents;
-    int64_t fCount;           // -1: no sample set
+    EventSample<Event> fSample;
     uint32_t* fCounts;        // [kBins][stride]
     size_t fCountsSize;
     int64_t fSlots;           // SMs x resident CTAs of kBinnedPairs; 0 until the first launch
     int fResident = 0;
 };
 
+// ---------------------------------------------------------------------------
+// Weighted binned event functors
+// ---------------------------------------------------------------------------
+constexpr int kWeightedMaxBins = 256;
+constexpr int64_t kWeightedMinChunk = 1024;
+constexpr int64_t kWeightedMaxChunks = 32;
+
+template <class F, class = void>
+struct IsWeightedBinnedFunctor : std::false_type {};
+template <class F>
+struct IsWeightedBinnedFunctor<F, decltype((void)F::kBins, (void)sizeof(typename F::Event), (void)&F::Weight)>
+    : std::true_type {};
+
+/// sums[b] of one point: a column of a [kBins][stride] table of doubles (stride 1
+/// on the host).
+class BinSums {
+public:
+    __host__ __device__ BinSums(const double* first, size_t stride) : fFirst(first), fStride(stride) {}
+    __host__ __device__ double operator[](int b) const { return fFirst[(size_t)b * fStride]; }
+
+private:
+    const double* fFirst;
+    size_t fStride;
+};
+
+template <class F>
+struct CheckWeightedFunctor {
+    static_assert(CheckBinnedFunctor<F>::value, "");
+    static_assert(F::kBins >= 1 && F::kBins <= kWeightedMaxBins,
+                  "F::kBins of a weighted binned functor must be between 1 and 256 (every point keeps a private "
+                  "FP64 histogram in shared memory: 32 points x 256 bins x 8 bytes = 64 KB per CTA)");
+    static_assert(std::is_same<decltype(std::declval<const F&>().Weight(std::declval<const typename F::Chain&>(),
+                                                                        std::declval<const typename F::Event&>())),
+                               double>::value,
+                  "F::Weight(chain, event) must return double");
+    static constexpr bool value = true;
+};
+
+/// Points (= threads) per CTA of kWeightedPairs: 128, 64 or 32, the most whose
+/// histograms, Points x kBins doubles, fit 48 KB; 32 above that (up to 64 KB).
+template <int Bins>
+struct WeightedShape {
+    static constexpr int kPoints = Bins * 128 * 8 <= 48 * 1024 ? 128 : Bins * 64 * 8 <= 48 * 1024 ? 64 : 32;
+};
+
+/// Events per chunk of the fixed summation order of weighted functors: N/32
+/// rounded up to whole tiles, at least kWeightedMinChunk.  A function of N only;
+/// a sample is at most kWeightedMaxChunks chunks.
+__host__ __device__ inline int64_t WeightedChunk(int64_t n) {
+    int64_t c = (n + kWeightedMaxChunks - 1) / kWeightedMaxChunks;
+    c = (c + kEventTile - 1) / kEventTile * kEventTile;
+    return c < kWeightedMinChunk ? kWeightedMinChunk : c;
+}
+__host__ __device__ inline int64_t WeightedChunks(int64_t n) {
+    const int64_t c = WeightedChunk(n);
+    return (n + c - 1) / c;
+}
+
+/// One CTA = P points (one thread each, P from kBins) x one chunk of events.  Tiles
+/// are staged as in kEventPairs.  Each thread keeps its point's histogram in shared
+/// memory, laid out [bin][P] so that a warp's 32 lanes hit consecutive 8-byte
+/// words, and adds the weight of every event whose Bin is in [0, kBins) to its bin
+/// in event order: a plain load, add and store, no atomics, since no other thread
+/// touches the column.  At the end of the chunk the column is written to
+/// partial[(chunk * kBins + bin) * stride + point], coalesced across lanes.
+///
+/// The staging loop is kEventPairs' own, as in kBinnedPairs (§4.10c of DESIGN.md).
+template <class F>
+__global__ void __launch_bounds__(WeightedShape<F::kBins>::kPoints)
+kWeightedPairs(const F* __restrict__ f, const typename F::Event* __restrict__ events, int64_t n, int64_t chunkEvents,
+               const double* __restrict__ x, int m, int dim, int pointTiles, int stride, double* __restrict__ partial) {
+    typedef typename F::Event Event;
+    constexpr int P = WeightedShape<F::kBins>::kPoints;
+    constexpr uint32_t kTileBytes = (uint32_t)(kEventTile * sizeof(Event));
+    extern __shared__ __align__(128) unsigned char smem[];
+    Event (*tiles)[kEventTile] = reinterpret_cast<Event (*)[kEventTile]>(smem);
+    __shared__ __align__(8) uint64_t bars[2];
+    const int tid = threadIdx.x;
+    double* hist = reinterpret_cast<double*>(smem + 2 * kTileBytes) + tid;   // this point's column, stride P
+    const int chunk = blockIdx.x / pointTiles;
+    const int point = (blockIdx.x - chunk * pointTiles) * P + tid;
+    const int64_t first = (int64_t)chunk * chunkEvents;
+    const int count = (int)min(chunkEvents, n - first);
+    const bool live = point < m;
+    typename F::Chain c;
+    if (live) c = f->Prepare(x + (size_t)point * dim, dim);
+    for (int b = 0; b < F::kBins; ++b) hist[b * P] = 0.0;
+
+    if (tid == 0) {
+        smcmc::mbarInit(&bars[0], 1);
+        smcmc::mbarInit(&bars[1], 1);
+        asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
+    }
+    __syncthreads();
+    const Event* src = events + first;
+    const int numTiles = (count + kEventTile - 1) / kEventTile;
+    if (tid == 0) {
+        smcmc::mbarExpectTx(&bars[0], kTileBytes);
+        smcmc::tmaLoad1D(tiles[0], src, kTileBytes, &bars[0]);
+    }
+    for (int t = 0; t < numTiles; ++t) {
+        const int buf = t & 1;
+        if (tid == 0 && t + 1 < numTiles) {
+            smcmc::mbarExpectTx(&bars[buf ^ 1], kTileBytes);
+            smcmc::tmaLoad1D(tiles[buf ^ 1], src + (size_t)(t + 1) * kEventTile, kTileBytes, &bars[buf ^ 1]);
+        }
+        smcmc::mbarWait(&bars[buf], (uint32_t)(t >> 1) & 1u);
+        const int len = min(kEventTile, count - t * kEventTile);
+        if (live) {
+#pragma unroll 2
+            for (int e = 0; e < len; ++e) {
+                const Event& ev = tiles[buf][e];
+                const int b = f->Bin(c, ev);
+                if ((unsigned)b < (unsigned)F::kBins) hist[b * P] += f->Weight(c, ev);
+            }
+        }
+        __syncthreads();
+    }
+    if (live)
+        for (int b = 0; b < F::kBins; ++b) partial[((size_t)chunk * F::kBins + b) * stride + point] = hist[b * P];
+}
+
+/// One thread per point: each bin's chunk partials added in chunk order, starting
+/// at 0.0, into the chunk-0 rows (partial[b * stride + point], in place: only this
+/// thread reads or writes the column), then Finish over them.  chunks = 0 (an empty
+/// sample) leaves every sum 0.0.
+template <class F>
+__global__ void __launch_bounds__(kThreads)
+kWeightedFinish(const F* __restrict__ f, double* __restrict__ partial, int chunks, int stride, int64_t n,
+                const double* __restrict__ x, int m, int dim, double* __restrict__ out) {
+    const int p = blockIdx.x * kThreads + threadIdx.x;
+    if (p >= m) return;
+    for (int b = 0; b < F::kBins; ++b) {
+        double s = 0.0;
+        for (int k = 0; k < chunks; ++k) s += partial[((size_t)k * F::kBins + b) * stride + p];
+        partial[(size_t)b * stride + p] = s;
+    }
+    out[p] = f->Finish(f->Prepare(x + (size_t)p * dim, dim), BinSums(partial + p, (size_t)stride), n);
+}
+
+/// sums[b] at one point, on the host, in the order of the header comment: the
+/// weights of the events with Bin(c, e) == b, added in event order within each
+/// chunk of WeightedChunk(n) events, the chunk sums added in chunk order.
+template <class F>
+void WeightedSumsHost(const F& f, const typename F::Event* events, int64_t n, const double* x, int dim, double* sums) {
+    static_assert(CheckWeightedFunctor<F>::value, "");
+    const typename F::Chain c = f.Prepare(x, dim);
+    const int64_t chunk = WeightedChunk(n);
+    std::vector<double> part(F::kBins);
+    for (int b = 0; b < F::kBins; ++b) sums[b] = 0.0;
+    for (int64_t first = 0; first < n; first += chunk) {
+        const int64_t last = first + chunk < n ? first + chunk : n;
+        for (int b = 0; b < F::kBins; ++b) part[b] = 0.0;
+        for (int64_t i = first; i < last; ++i) {
+            const int b = f.Bin(c, events[i]);
+            if ((unsigned)b < (unsigned)F::kBins) part[b] += f.Weight(c, events[i]);
+        }
+        for (int b = 0; b < F::kBins; ++b) sums[b] += part[b];
+    }
+}
+
+/// The value of a weighted binned functor at one point, on the host:
+/// Finish(c, sums, n) over WeightedSumsHost.
+template <class F>
+double WeightedBinnedLikelihoodHost(const F& f, const typename F::Event* events, int64_t n, const double* x, int dim) {
+    std::vector<double> sums(F::kBins);
+    WeightedSumsHost(f, events, n, x, dim, sums.data());
+    return f.Finish(f.Prepare(x, dim), BinSums(sums.data(), 1), n);
+}
+
+/// The device copies of one weighted binned functor and its sample, the partial
+/// sums, and the launch table.  One WeightedBinnedBinding serves one engine (the
+/// partial sums are used on that engine's stream).
+template <class F>
+class WeightedBinnedBinding {
+    static_assert(CheckWeightedFunctor<F>::value, "");
+
+public:
+    typedef typename F::Event Event;
+    static constexpr int kPoints = WeightedShape<F::kBins>::kPoints;
+    static constexpr size_t kSmemBytes = 2 * kEventTile * sizeof(Event) + (size_t)F::kBins * kPoints * sizeof(double);
+
+    WeightedBinnedBinding() : fDevice(nullptr), fPartial(nullptr), fPartialSize(0), fResident(0) {}
+    ~WeightedBinnedBinding() {
+        if (fDevice) cudaFree(fDevice);
+        if (fPartial) cudaFree(fPartial);
+    }
+    WeightedBinnedBinding(const WeightedBinnedBinding&) = delete;
+    WeightedBinnedBinding& operator=(const WeightedBinnedBinding&) = delete;
+
+    /// Copy the sample to the GPU.  n = 0 is an empty sample (all sums 0).
+    void SetEvents(const Event* events, int64_t n) { fSample.Set(events, n); }
+    bool HasEvents() const { return fSample.Has(); }
+    int64_t GetEventCount() const { return fSample.Count(); }
+
+    /// Copy the functor to the GPU (again).
+    void Upload(const F& host) {
+        if (!fDevice) Check(cudaMalloc((void**)&fDevice, sizeof(F)));
+        Check(cudaMemcpy(fDevice, &host, sizeof(F), cudaMemcpyHostToDevice));
+    }
+    /// Upload the functor and register with an engine created with SMCMC_LLH_USER;
+    /// the sample must have been set.
+    void Bind(smcmc_engine* e, const F& host) {
+        if (!HasEvents()) throw std::logic_error("weighted binned functor: no event sample set (SetEvents) before Bind");
+        Upload(host);
+        smcmc_user_ops ops;
+        ops.struct_size = sizeof ops;
+        ops.reserved_ = 0;
+        ops.ctx = this;
+        ops.likelihood = &WeightedBinnedBinding::LaunchLikelihood;
+        ops.gradient = nullptr;                       // a binned likelihood is piecewise constant
+        const int rc = smcmc_user_set_ops(e, &ops);
+        if (rc != SMCMC_OK) throw std::logic_error(smcmc_last_error(e));
+    }
+    /// Bind with a sample given as raw bytes (a C entry point of a user library):
+    /// itemsize must be sizeof(Event).
+    void Bind(smcmc_engine* e, const F& host, const void* events, int64_t n, size_t itemsize) {
+        if (itemsize != sizeof(Event))
+            throw std::invalid_argument("event item size " + std::to_string(itemsize) + " != sizeof(Event) " +
+                                        std::to_string(sizeof(Event)));
+        SetEvents(static_cast<const Event*>(events), n);
+        Bind(e, host);
+    }
+
+    /// The weighted histograms of the functor last uploaded at m host points
+    /// x[m][dim]: out[p * kBins + b], synchronously, the sums Finish receives.
+    void Sums(const double* x, int m, int dim, double* out) {
+        if (!HasEvents() || !fDevice) throw std::logic_error("weighted binned functor: Sums before SetEvents and Upload");
+        if (m < 1 || dim < 1 || !x || !out) throw std::invalid_argument("Sums: bad point array");
+        const int stride = (m + 31) / 32 * 32;
+        const size_t need = Scratch(m);
+        double* dx = nullptr;
+        double* dp = nullptr;
+        double* dv = nullptr;
+        std::vector<double> table((size_t)F::kBins * stride);
+        cudaError_t rc = cudaMalloc((void**)&dx, (size_t)m * dim * sizeof(double));
+        if (rc == cudaSuccess) rc = cudaMalloc((void**)&dp, need * sizeof(double));
+        if (rc == cudaSuccess) rc = cudaMalloc((void**)&dv, (size_t)m * sizeof(double));
+        if (rc == cudaSuccess) rc = cudaMemcpy(dx, x, (size_t)m * dim * sizeof(double), cudaMemcpyHostToDevice);
+        if (rc == cudaSuccess) rc = (cudaError_t)Evaluate(dx, m, dim, dp, dv, 0);
+        if (rc == cudaSuccess) rc = cudaMemcpy(table.data(), dp, table.size() * sizeof(double), cudaMemcpyDeviceToHost);
+        if (dx) cudaFree(dx);
+        if (dp) cudaFree(dp);
+        if (dv) cudaFree(dv);
+        Check(rc);
+        for (int p = 0; p < m; ++p)
+            for (int b = 0; b < F::kBins; ++b) out[(size_t)p * F::kBins + b] = table[(size_t)b * stride + p];
+    }
+    /// Resident CTAs of kWeightedPairs per SM (queried at the first launch; 0 before it).
+    int ResidentCtas() const { return fResident; }
+
+private:
+    static void Check(cudaError_t rc) {
+        if (rc != cudaSuccess) throw std::runtime_error(std::string("CUDA: ") + cudaGetErrorString(rc));
+    }
+    // doubles of partial sums for m points: [max(chunks, 1)][kBins][stride]
+    size_t Scratch(int m) const {
+        const int64_t chunks = WeightedChunks(fSample.Count());
+        return (size_t)(chunks > 1 ? chunks : 1) * F::kBins * (size_t)((m + 31) / 32 * 32);
+    }
+    // the sums into partial's chunk-0 rows and the values into out, on stream s
+    int Evaluate(const double* x, int m, int dim, double* partial, double* out, cudaStream_t s) {
+        cudaError_t rc;
+        if (fResident == 0) {                         // kWeightedPairs' shared memory and occupancy, once
+            if (kSmemBytes > 48 * 1024 &&
+                (rc = cudaFuncSetAttribute(kWeightedPairs<F>, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                                           (int)kSmemBytes)) != cudaSuccess)
+                return (int)rc;
+            if ((rc = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&fResident, kWeightedPairs<F>, kPoints,
+                                                                    kSmemBytes)) != cudaSuccess)
+                return (int)rc;
+            if (fResident < 1) return (int)cudaErrorInvalidConfiguration;
+        }
+        const int64_t n = fSample.Count();
+        const int chunks = (int)WeightedChunks(n);
+        const int stride = (m + 31) / 32 * 32;
+        const int pointTiles = (m + kPoints - 1) / kPoints;
+        if (chunks > 0)
+            kWeightedPairs<F><<<(unsigned)chunks * (unsigned)pointTiles, kPoints, kSmemBytes, s>>>(
+                fDevice, fSample.Data(), n, WeightedChunk(n), x, m, dim, pointTiles, stride, partial);
+        kWeightedFinish<F><<<(m + kThreads - 1) / kThreads, kThreads, 0, s>>>(fDevice, partial, chunks, stride, n, x, m,
+                                                                             dim, out);
+        return (int)cudaGetLastError();
+    }
+    static int LaunchLikelihood(void* ctx, const double* x, int m, int n, double* out, void* stream) {
+        WeightedBinnedBinding* b = static_cast<WeightedBinnedBinding*>(ctx);
+        cudaStream_t s = (cudaStream_t)stream;
+        const size_t need = b->Scratch(m);
+        if (need > b->fPartialSize) {                 // grows only: stream-ordered on the engine's stream
+            if (b->fPartial) {
+                cudaError_t rc = cudaFreeAsync(b->fPartial, s);
+                if (rc != cudaSuccess) return (int)rc;
+                b->fPartial = nullptr;
+                b->fPartialSize = 0;
+            }
+            cudaError_t rc = cudaMallocAsync((void**)&b->fPartial, need * sizeof(double), s);
+            if (rc != cudaSuccess) return (int)rc;
+            b->fPartialSize = need;
+        }
+        return b->Evaluate(x, m, n, b->fPartial, out, s);
+    }
+
+    F* fDevice;
+    EventSample<Event> fSample;
+    double* fPartial;         // [chunks][kBins][stride]
+    size_t fPartialSize;
+    int fResident;            // resident CTAs of kWeightedPairs per SM; 0 until the first launch
+};
+
 }  // namespace smcmc_user
 
 // The sampler side: a likelihood class WITHOUT a built-in id (no kDeviceLikelihood
 // member) is a user device functor; one with a nested Event type is an event functor,
-// binned when it also has kBins.
+// binned when it also has kBins, weighted binned when it also has Weight.
 namespace sMCMC {
 namespace detail {
 template <class L, class Enable>
@@ -879,8 +1228,14 @@ struct DeviceBinding<L, typename std::enable_if<smcmc_user::IsEventFunctor<L>::v
     : EventSampleBinding<L, smcmc_user::EventBinding<L> > {};
 // a binned likelihood is piecewise constant: TSimpleHMC refuses it (kHmcUsable)
 template <class L>
-struct DeviceBinding<L, typename std::enable_if<smcmc_user::IsBinnedFunctor<L>::value>::type>
+struct DeviceBinding<L, typename std::enable_if<smcmc_user::IsBinnedFunctor<L>::value &&
+                                                !smcmc_user::IsWeightedBinnedFunctor<L>::value>::type>
     : EventSampleBinding<L, smcmc_user::BinnedBinding<L> > {
+    static constexpr bool kHmcUsable = false;
+};
+template <class L>
+struct DeviceBinding<L, typename std::enable_if<smcmc_user::IsWeightedBinnedFunctor<L>::value>::type>
+    : EventSampleBinding<L, smcmc_user::WeightedBinnedBinding<L> > {
     static constexpr bool kHmcUsable = false;
 };
 }  // namespace detail
