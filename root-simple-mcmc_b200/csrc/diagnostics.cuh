@@ -10,6 +10,7 @@
 //
 //   pooled : double[1 + n + n(n+1)/2]   (count, sum x, packed sum x x^T) over chains and steps (kPoolAccumulate)
 //   s1, s2 : double[E][n]               per-chain sum x, sum x^2
+//   chainCount: double[E]               per-chain number of steps behind s1, s2 (steps it was running)
 //   ring   : double[depth][E][n]        the last `depth` accepted points of every chain
 //   lagProd: double[nlags][n]           sum over chains and steps of x_i(t) x_i(t - lag)
 //   lagCount: double[nlags]             number of (chain, step) pairs behind each lagProd row
@@ -24,6 +25,7 @@ struct DiagArrays {
     double* pooled;
     double* s1;
     double* s2;
+    double* chainCount;
     double* ring;
     double* lagProd;
     double* lagCount;
@@ -44,6 +46,7 @@ kDiagChains(const double* __restrict__ x, const ChainScalars* __restrict__ sc, i
     if (live) {
         d.s1[k] += v;
         d.s2[k] += v * v;
+        if (k == (size_t)c * n) d.chainCount[c] += 1.0;
     }
     if (d.depth > 0) d.ring[(size_t)slot * chains * n + k] = v;     // NaN marks a chain that is not running
 }

@@ -218,7 +218,7 @@ struct smcmc_engine {
     int diagDepth = 0;
     long long diagFills = 0;
     std::vector<int> diagLags;
-    DeviceBuffer<double> diagPooled, diagS1, diagS2, diagRing, diagLagProd, diagLagCount;
+    DeviceBuffer<double> diagPooled, diagS1, diagS2, diagChainCount, diagRing, diagLagProd, diagLagCount;
     DeviceBuffer<int> diagLagsDev;
 
     DiagArrays diagArrays() {
@@ -226,6 +226,7 @@ struct smcmc_engine {
         d.pooled = diagPooled.get();
         d.s1 = diagS1.get();
         d.s2 = diagS2.get();
+        d.chainCount = diagChainCount.get();
         d.ring = diagRing.get();
         d.lagProd = diagLagProd.get();
         d.lagCount = diagLagCount.get();
@@ -239,6 +240,7 @@ struct smcmc_engine {
         CUDA_CHECK(cudaMemsetAsync(diagPooled.get(), 0, poolStatCount() * sizeof(double), stream));
         CUDA_CHECK(cudaMemsetAsync(diagS1.get(), 0, En * sizeof(double), stream));
         CUDA_CHECK(cudaMemsetAsync(diagS2.get(), 0, En * sizeof(double), stream));
+        CUDA_CHECK(cudaMemsetAsync(diagChainCount.get(), 0, E() * sizeof(double), stream));
         if (!diagLags.empty()) {
             CUDA_CHECK(cudaMemsetAsync(diagLagProd.get(), 0, diagLags.size() * n() * sizeof(double), stream));
             CUDA_CHECK(cudaMemsetAsync(diagLagCount.get(), 0, diagLags.size() * sizeof(double), stream));
@@ -2177,6 +2179,7 @@ int smcmc_diag_enable(smcmc_engine* e, int max_lag) {
         e->diagPooled.reserve(e->poolStatCount());
         e->diagS1.reserve(En);
         e->diagS2.reserve(En);
+        e->diagChainCount.reserve(e->E());
         if (max_lag > 0) {
             e->diagRing.reserve((size_t)max_lag * En);
             e->diagLagProd.reserve(e->diagLags.size() * e->n());
@@ -2210,10 +2213,11 @@ int smcmc_diag_get(smcmc_engine* e, const smcmc_diag_result* out) {
         if (!out) throw Error(SMCMC_ERR_INVALID_ARGUMENT, "null result");
         const size_t E = e->E(), n = e->n(), nl = e->diagLags.size();
         CUDA_CHECK(cudaStreamSynchronize(e->stream));
-        std::vector<double> pooled(e->poolStatCount()), s1(E * n), s2(E * n), lp(nl * n), lc(nl);
+        std::vector<double> pooled(e->poolStatCount()), s1(E * n), s2(E * n), cc(E), lp(nl * n), lc(nl);
         CUDA_CHECK(cudaMemcpy(pooled.data(), e->diagPooled.get(), pooled.size() * 8, cudaMemcpyDeviceToHost));
         CUDA_CHECK(cudaMemcpy(s1.data(), e->diagS1.get(), s1.size() * 8, cudaMemcpyDeviceToHost));
         CUDA_CHECK(cudaMemcpy(s2.data(), e->diagS2.get(), s2.size() * 8, cudaMemcpyDeviceToHost));
+        CUDA_CHECK(cudaMemcpy(cc.data(), e->diagChainCount.get(), cc.size() * 8, cudaMemcpyDeviceToHost));
         if (nl) {
             CUDA_CHECK(cudaMemcpy(lp.data(), e->diagLagProd.get(), lp.size() * 8, cudaMemcpyDeviceToHost));
             CUDA_CHECK(cudaMemcpy(lc.data(), e->diagLagCount.get(), lc.size() * 8, cudaMemcpyDeviceToHost));
@@ -2241,8 +2245,9 @@ int smcmc_diag_get(smcmc_engine* e, const smcmc_diag_result* out) {
                 double W = 0.0, m1 = 0.0, m2 = 0.0;
                 size_t M = 0;
                 for (size_t c = 0; c < E; ++c) {
+                    // only chains that ran at every accumulated step (a chain that sits at 0 runs too)
+                    if (cc[c] != N) continue;
                     const double a = s1[c * n + i], b = s2[c * n + i];
-                    if (a == 0.0 && b == 0.0) continue;                    // chain not running
                     const double cm = a / N;
                     W += (b - N * cm * cm) / (N - 1.0);
                     m1 += cm;
